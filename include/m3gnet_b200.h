@@ -422,6 +422,20 @@ int m3g_readout_fwd_bwd(const float* x, const float* W0dT, const float* b0d, con
 /* forces = -g_pos; stresses (B,6) = Voigt(sum_i pos_i (x) F_i)/|det lattice| */
 int m3g_forces_virial(const float* pos, const float* g_pos, const float* lattice, const int32_t* atom_ptr,
                       int64_t N, int64_t B, float* forces, float* stresses, void* stream);
+/* Cell stress (extension, no reference counterpart; the reference's only stress is the origin-dependent virial row of
+ * nn/gradient.py:25-64 above).  sigma (B,3,3) row-major, eV/A^3:
+ *   sigma_b[a][c] = (1/V_b) sum_{e in structure b} v_e[a] g_e[c],   g_e = g_vec4.xyz + (g_vec4.w + g_dist)·v/r,
+ * i.e. (1/V) dE_b/d(eps_ac) at eps = 0 for positions and lattice rows deformed as r -> r (I + eps); V_b = |det lattice_b|.
+ * Same bond-gradient inputs as m3g_geometry_bwd (g_vec4 / g_dist may be NULL); vec4 and its gradient may be in scaled
+ * lengths (v (x) dE/dv does not depend on the length unit), lattice must be in A.  ASE convention: Voigt order
+ * [xx, yy, zz, yz, xz, xy] of sigma is ASE's "stress" (pressure = -tr(sigma)/3; positive = tensile).  The bonds of
+ * structure b are edge_ptr[atom_ptr[b]] .. edge_ptr[atom_ptr[b+1]]; structures without bonds get sigma = 0.
+ * Deterministic: float64 partial sums over fixed 2048-bond chunks, then a fixed-order sum per structure (two launches,
+ * no atomics).  work: m3g_bond_virial_work_elems(E, B) doubles of caller-owned scratch. */
+int64_t m3g_bond_virial_work_elems(int64_t E, int64_t B);
+int m3g_bond_virial(const float* vec4, const float* g_vec4, const float* g_dist, const int32_t* edge_ptr,
+                    const int32_t* atom_ptr, int64_t E, int64_t B, const float* lattice, double* work, float* sigma,
+                    void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Domain decomposition helpers (new; nothing in the reference — nn/gradient.py:26 TODO)

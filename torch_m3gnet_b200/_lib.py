@@ -87,7 +87,7 @@ LIB = _Library()
 CALLS = 0
 LAUNCHES = 0
 _KERNELS_PER_CALL = {"exclusive_scan_i32": 3, "csr_by_key": 7, "check_sorted": 2, "csr_is_symmetric": 2,
-                     "forces_virial": 2}
+                     "forces_virial": 2, "bond_virial": 2}
 # when set to a dict, every call is bracketed by CUDA events on the launching stream: {name: [(start, end), ...]}
 PROFILE = None
 
@@ -189,6 +189,10 @@ def _launch(name, fn, conv, index):
 
 def scan_work_elems(n: int) -> int:
     return int(LIB.load().m3g_scan_work_elems(n))
+
+
+def bond_virial_work_elems(E: int, B: int) -> int:
+    return int(LIB.load().m3g_bond_virial_work_elems(E, B))
 
 
 def tb_atom_capacity() -> int:

@@ -312,6 +312,106 @@ __global__ void virial_kernel(const float* __restrict__ pos, const float* __rest
   }
 }
 
+// Cell stress as the strain derivative of the energy (no reference counterpart): W_b = sum_{e in b} v_e (x) g_e with
+// g_e = g_vec4.xyz + (g_vec4.w + g_dist) v/r, sigma_b = W_b / |det lattice_b|.  Deterministic two-stage reduction in
+// float64.  Stage 1: block c owns the bonds [c*CH, (c+1)*CH) and writes one partial per (structure b, chunk c) segment
+// at slot b + c (both indices are non-decreasing along the bonds and never repeat together, so slots are distinct).
+// Stage 2: one warp per structure sums its slots b + c0 .. b + c1 in a fixed order.
+constexpr int kVirialThreads = 256;
+constexpr int kVirialChunk = 2048;
+
+__device__ __forceinline__ int64_t structure_first_bond(const int32_t* edge_ptr, const int32_t* atom_ptr, int64_t b) {
+  return edge_ptr[atom_ptr[b]];
+}
+
+__global__ void __launch_bounds__(kVirialThreads) bond_virial_partial_kernel(
+    const float4* __restrict__ vec4, const float4* __restrict__ g_vec4, const float* __restrict__ g_dist,
+    const int32_t* __restrict__ edge_ptr, const int32_t* __restrict__ atom_ptr, int64_t E, int64_t B,
+    double* __restrict__ part) {
+  __shared__ double red[kVirialThreads / 32][9];
+  __shared__ int64_t seg[2];
+  const int64_t c = blockIdx.x;
+  const int64_t c_begin = c * kVirialChunk;
+  const int64_t c_end = min(c_begin + (int64_t)kVirialChunk, E);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int64_t start = c_begin;
+  while (start < c_end) {
+    if (threadIdx.x == 0) {
+      // structure of bond `start`: last b with first_bond(b) <= start (empty structures share their first bond with
+      // the next one, so the search lands on the structure that owns the bond)
+      int64_t lo = 0, hi = B - 1;
+      while (lo < hi) {
+        int64_t mid = (lo + hi + 1) >> 1;
+        if (structure_first_bond(edge_ptr, atom_ptr, mid) <= start) lo = mid;
+        else hi = mid - 1;
+      }
+      seg[0] = lo;
+      seg[1] = min((int64_t)edge_ptr[atom_ptr[lo + 1]], c_end);
+    }
+    __syncthreads();
+    const int64_t b = seg[0], stop = seg[1];
+    double w[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) w[k] = 0.0;
+    for (int64_t e = start + threadIdx.x; e < stop; e += kVirialThreads) {
+      const float4 v = vec4[e];
+      const float4 g = g_vec4 ? g_vec4[e] : make_float4(0.f, 0.f, 0.f, 0.f);
+      const float s = (g.w + (g_dist ? g_dist[e] : 0.0f)) / v.w;
+      const double ge[3] = {(double)(g.x + s * v.x), (double)(g.y + s * v.y), (double)(g.z + s * v.z)};
+      const double vv[3] = {(double)v.x, (double)v.y, (double)v.z};
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int k = 0; k < 3; ++k) w[3 * a + k] += vv[a] * ge[k];
+    }
+#pragma unroll
+    for (int k = 0; k < 9; ++k) {
+      double t = w[k];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+      if (lane == 0) red[warp][k] = t;
+    }
+    __syncthreads();
+    if (threadIdx.x < 9) {
+      double t = 0.0;
+#pragma unroll
+      for (int q = 0; q < kVirialThreads / 32; ++q) t += red[q][threadIdx.x];
+      part[(b + c) * 9 + threadIdx.x] = t;
+    }
+    start = stop;
+    __syncthreads();  // seg / red are rewritten by the next segment
+  }
+}
+
+__global__ void bond_virial_finish_kernel(const double* __restrict__ part, const int32_t* __restrict__ edge_ptr,
+                                          const int32_t* __restrict__ atom_ptr, const float* __restrict__ lattice,
+                                          int64_t B, float* __restrict__ sigma) {
+  const int64_t b = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const int64_t s = edge_ptr[atom_ptr[b]], t = edge_ptr[atom_ptr[b + 1]];
+  double w[9];
+#pragma unroll
+  for (int k = 0; k < 9; ++k) w[k] = 0.0;
+  if (t > s) {
+    const int64_t c0 = s / kVirialChunk, c1 = (t - 1) / kVirialChunk;
+    for (int64_t c = c0 + lane; c <= c1; c += 32)
+#pragma unroll
+      for (int k = 0; k < 9; ++k) w[k] += part[(b + c) * 9 + k];
+  }
+  const float* Lm = lattice + b * 9;
+  const double vol = fabs((double)Lm[0] * ((double)Lm[4] * Lm[8] - (double)Lm[5] * Lm[7]) +
+                          (double)Lm[1] * ((double)Lm[5] * Lm[6] - (double)Lm[3] * Lm[8]) +
+                          (double)Lm[2] * ((double)Lm[3] * Lm[7] - (double)Lm[4] * Lm[6]));
+#pragma unroll
+  for (int k = 0; k < 9; ++k) {
+    double x = w[k];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+    if (lane == 0) sigma[b * 9 + k] = (float)(x / vol);
+  }
+}
+
 }  // namespace m3g
 
 using namespace m3g;
@@ -436,6 +536,26 @@ int m3g_forces_virial(const float* pos, const float* g_pos, const float* lattice
   if (B > 0)
     virial_kernel<<<blocks_for(B * 32, 128), 128, 0, as_stream(stream)>>>(pos, forces, lattice, atom_ptr, B, stresses);
   M3G_LAUNCH_CHECK("m3g_forces_virial");
+  return M3G_OK;
+}
+
+int64_t m3g_bond_virial_work_elems(int64_t E, int64_t B) {
+  return 9 * (B + (E + kVirialChunk - 1) / kVirialChunk);
+}
+
+int m3g_bond_virial(const float* vec4, const float* g_vec4, const float* g_dist, const int32_t* edge_ptr,
+                    const int32_t* atom_ptr, int64_t E, int64_t B, const float* lattice, double* work, float* sigma,
+                    void* stream) {
+  if (B == 0) return M3G_OK;
+  M3G_REQUIRE(edge_ptr && atom_ptr && lattice && work && sigma, "m3g_bond_virial: null pointer");
+  M3G_REQUIRE(E == 0 || vec4, "m3g_bond_virial: null vec4");
+  const int64_t chunks = (E + kVirialChunk - 1) / kVirialChunk;
+  // a chunk-less batch (no bonds) still takes one (empty) stage-1 block: two launches per call, always
+  bond_virial_partial_kernel<<<chunks > 0 ? chunks : 1, kVirialThreads, 0, as_stream(stream)>>>(
+      (const float4*)vec4, (const float4*)g_vec4, g_dist, edge_ptr, atom_ptr, E, B, work);
+  bond_virial_finish_kernel<<<blocks_for(B * 32, 128), 128, 0, as_stream(stream)>>>(work, edge_ptr, atom_ptr, lattice,
+                                                                                    B, sigma);
+  M3G_LAUNCH_CHECK("m3g_bond_virial");
   return M3G_OK;
 }
 

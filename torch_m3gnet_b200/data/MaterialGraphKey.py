@@ -18,7 +18,13 @@ _TARGET = {
     "TOTAL_ENERGY": "total_energy", "FORCES": "forces", "STRESSES": "stresses",
 }
 _BATCH = {"BATCH": "batch"}
+# extensions with no reference counterpart
+_EXTENSION = {
+    # (B,3,3) eV/A^3: sigma = (1/V) dE/d(strain), ASE's stress convention; filled when Gradient.compute_stress is set.
+    # Not the reference's STRESSES row (sum_i pos_i (x) F_i / V), which keeps its meaning.
+    "CELL_STRESS": "cell_stress",
+}
 
-ALL_KEYS = {**_INPUT, **_DERIVED, **_TARGET, **_BATCH}
+ALL_KEYS = {**_INPUT, **_DERIVED, **_TARGET, **_BATCH, **_EXTENSION}
 globals().update(ALL_KEYS)
 __all__ = list(ALL_KEYS)

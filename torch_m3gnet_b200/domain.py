@@ -226,7 +226,14 @@ class EmulatedHaloFn(torch.autograd.Function):
         return (None,) + tuple(g_in)
 
 
+def _no_cell_stress(model):
+    if getattr(model, "compute_stress", False):
+        raise NotImplementedError("the cell stress (compute_stress) is not implemented for domain-decomposed cells: "
+                                  "ghost bonds and the cross-rank reduction are not handled")
+
+
 def _modules_of(model):
+    _no_cell_stress(model)
     seq = model.model if hasattr(model, "model") else model
     mods = list(seq)
     last_conv = max(i for i, m in enumerate(mods) if isinstance(m, M3GNetConv))
@@ -317,6 +324,8 @@ class DomainStep:
 
         from torch_m3gnet_b200 import engine as E
         from torch_m3gnet_b200.data.material_graph import get_plan
+
+        _no_cell_stress(model)
 
         self.dist, self.E, self.group = dist, E, group
         self.model, self.dbatch = model, dbatch

@@ -286,21 +286,40 @@ class StepEngine:
         if rc != 0:
             raise RuntimeError(f"m3g_step_run failed ({rc}): {lib.m3g_last_error().decode()}")
 
-    def launches(self, with_angles: bool = True) -> int:
+    def launches(self, with_angles: bool = True, stress: bool = False) -> int:
         """Kernel launches of one full step (for bench.py's gpu_launches): prologue 7 (6 when e0 is formed inside the first three-body edge update; +1 for the cos output) + one
         radial table per distinct constant set, 6 per block forward, 2 for the readout with its adjoint, 7 per block
-        backward (3 for block 0, whose node-feature gradient is dead; +1 per block with the split three-body adjoint), 4 in the epilogue, 2 for forces + virial."""
+        backward (3 for block 0, whose node-feature gradient is dead; +1 per block with the split three-body adjoint), 4 in the epilogue, 2 for forces + virial;
+        +2 for the cell stress (m3g_bond_virial) when ``stress`` is set."""
         n = self.n_blocks
         tables = len({t._packed.get()["consts_key"] for t in self.tbs})
         from torch_m3gnet_b200.nn import interaction
 
         return (7 - int(interaction.TB_SPLIT and FUSE_E0) + int(with_angles) + tables + (6 + int(interaction.TB_SPLIT)) * n + 2
-                + (7 * n - 4 + int(interaction.TB_BWD_SPLIT) * n) + 4 + 2)
+                + (7 * n - 4 + int(interaction.TB_BWD_SPLIT) * n) + 4 + 2 + 2 * int(stress))
 
-    def run(self, graph, plan):
+    @staticmethod
+    def cell_stress(keep) -> torch.Tensor:
+        """sigma (B,3,3) from the bond vectors and bond gradients the epilogue fed to m3g_geometry_bwd (still in the
+        scratch after the forces phase); volume from the unscaled lattice."""
+        from torch_m3gnet_b200.nn._functions import cell_stress
+
+        scratch, off, plan = keep["scratch"], keep["off"], keep["plan"]
+        E = plan.E
+
+        def view(name, n):
+            return scratch[off[name]:off[name] + n]
+
+        lat = keep["inputs"][1]
+        with torch.cuda.device(scratch.device):
+            return cell_stress(view("vec4", 4 * E), view("g_vec4", 4 * E), view("g_dist", E), plan, lat)
+
+    def run(self, graph, plan, stress: bool = False):
         desc, keep = self.prepare(graph, plan)
         self.run_phases(desc, 0, phase_forces(self.n_blocks), graph[K.POS].device)
-        _lib.LAUNCHES += self.launches(keep["out"][K.TRIPLET_ANGLES] is not None)
+        _lib.LAUNCHES += self.launches(keep["out"][K.TRIPLET_ANGLES] is not None)  # the stress call counts its own
+        if stress:
+            keep["out"][K.CELL_STRESS] = self.cell_stress(keep)
         for k, v in keep["out"].items():
             graph[k] = v
         # the scratch (activations, adjoints) goes back to the caching allocator here; stream order makes that safe

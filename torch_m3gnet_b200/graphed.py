@@ -3,7 +3,8 @@ relaxation between neighbour-list rebuilds).
 
 For small systems the step is launch-bound: ~60 kernel launches plus the autograd bookkeeping of a 32-atom cell cost
 far more host time than GPU time.  ``GraphedStep`` captures one ``model(batch)`` call — forward kernels, the hand-written
-adjoint kernels driven by ``torch.autograd.grad`` and the force / virial assembly — into a CUDA graph and replays it:
+adjoint kernels driven by ``torch.autograd.grad``, the force / virial assembly and, when the model's
+``compute_stress`` is set, the cell stress (``CELL_STRESS``) — into a CUDA graph and replays it:
 
     step = GraphedStep(model, batch)          # warm-up + capture (positions / lattice are static buffers)
     out = step()                              # replay with the captured positions
@@ -44,7 +45,8 @@ class GraphedStep:
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             out = model(batch)
-        self.out: Dict[str, torch.Tensor] = {k: out[k] for k in _KEYS}
+        keys = _KEYS + ((K.CELL_STRESS,) if getattr(model, "compute_stress", False) else ())
+        self.out: Dict[str, torch.Tensor] = {k: out[k] for k in keys}
         # the captured launches hold the device addresses of the packed weight images / constant tables that existed
         # at capture time; remember what they were made from so that a later parameter edit is noticed
         self._weights = self._weight_signature()

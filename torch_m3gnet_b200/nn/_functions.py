@@ -81,7 +81,10 @@ class GeometryFn(Function):
     """nn/invariant.py:20-59 → (vec4 (E,4) = (v, |v|), distances (E), clamped cos (T))."""
 
     @staticmethod
-    def forward(ctx, pos, lattice, plan, tri_index):
+    def forward(ctx, pos, lattice, plan, tri_index, strain=None, cell=None):
+        """``strain`` (optional, (B,3,3) zeros requiring grad): a handle whose gradient is the cell stress
+        sigma = (1/V) dE/d(strain) of ``cell_stress`` (``cell`` = the unscaled lattice, for V); it does not enter the
+        forward values."""
         ctx.set_materialize_grads(False)
         pos = pos.contiguous()
         lattice = lattice.contiguous()
@@ -96,6 +99,7 @@ class GeometryFn(Function):
             call("angles_fwd", vec4, tri_index, T, cos)
         ctx.plan = plan
         ctx.tri_index = tri_index
+        ctx.cell = None if strain is None else cell.detach().reshape(-1, 3, 3).contiguous()
         ctx.save_for_backward(vec4)
         return vec4, dist, cos
 
@@ -110,7 +114,22 @@ class GeometryFn(Function):
             call("angles_bwd", vec4, ctx.tri_index, g_cos.contiguous(), plan.T, g_vec4)
         g_pos = _empty((plan.N, 3), vec4)
         call("geometry_bwd", vec4, g_vec4, g_dist, plan.edge_ptr, plan.in_ptr, plan.in_perm, plan.N, 1.0, g_pos)
-        return g_pos, None, None, None
+        g_strain = None
+        if ctx.cell is not None and ctx.needs_input_grad[4]:
+            g_strain = cell_stress(vec4, g_vec4, g_dist, plan, ctx.cell)
+        return g_pos, None, None, None, g_strain, None
+
+
+def cell_stress(vec4, g_vec4, g_dist, plan, cell):
+    """sigma (B,3,3) = (1/V) sum_{bonds of b} v (x) dE/dv  (m3g_bond_virial): the strain derivative of the energy per
+    structure in eV/A^3, from the bond-gradient inputs of m3g_geometry_bwd (g_vec4 / g_dist may be None); ``cell`` is
+    the (B,3,3) lattice in A."""
+    B = plan.B
+    work = torch.empty(max(_lib.bond_virial_work_elems(plan.E, B), 1), dtype=torch.float64, device=vec4.device)
+    sigma = torch.empty((B, 3, 3), dtype=torch.float32, device=vec4.device)
+    call("bond_virial", vec4, _c(g_vec4), _c(g_dist), plan.edge_ptr, plan.atom_ptr, plan.E, B,
+         cell.to(torch.float32).contiguous(), work, sigma)
+    return sigma
 
 
 class RadialFn(Function):
