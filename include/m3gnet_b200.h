@@ -438,6 +438,34 @@ int m3g_bond_virial(const float* vec4, const float* g_vec4, const float* g_dist,
                     void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Batched FIRE relaxation step (csrc/relax.cu; extension, no reference counterpart): one step of calculator.py::Fire
+ * for every running structure of a ragged batch, each with its own FIRE state.  Per structure b (rows
+ * atom_ptr[b] .. atom_ptr[b+1]) whose status[b] == 0:
+ *   - generalised forces g: forces (N,3) f32 as they are, or with the cell filter (sigma != NULL; ASE UnitCellFilter
+ *     as Fire(relax_cell=True)): D = solve(L0_b, lattice_b)^T, atom rows F D, 3 cell rows
+ *     -|det lattice_b| (sigma_b + pressure I) D^-T / cell_factor[b];
+ *   - fmax[b] = max row |g| (+inf and status 3 = failed if any g is not finite); fmax[b] < fmax_target -> status 1
+ *     (converged); else n_steps[b] >= max_steps -> status 2 (not converged); otherwise one FIRE step with Fire's
+ *     parameters (P = g.v > 0: v = (1-a) v + a|v| g/max(|g|,1e-30), dt / a updated after n_min positive steps;
+ *     else v = 0, a = a_start, dt *= f_dec), v += dt g, dr = dt v clipped to |dr| <= max_move (norm over the
+ *     structure's rows), n_steps[b] += 1;
+ *   - without the cell filter pos (N,3) += dr; with it the generalised positions x (N,3) and xc (B,3,3) (= cell_factor
+ *     D; initially pos and cell_factor I) get dr, and pos = x Dn^T, lattice_b = L0_b Dn^T with Dn = xc_b / cell_factor[b];
+ *   - e_frame[b] = energy[b] and sigma_frame = sigma (f64, cell filter only) of the frame just checked (e_frame may be
+ *     NULL).  Together with pos / lattice / fmax these are the values of the frame at which a structure stopped.
+ * Velocities v (N,3), vc (B,3,3); dt, a (B) f64; n_pos, n_steps, status (B) int32; L0, lattice (B,3,3) f64 row-major.
+ * Structures with status != 0 are not touched.  Without the cell filter x, xc, vc, L0, lattice, cell_factor and
+ * sigma_frame are not read (may be NULL).  One launch, one 256-thread block per structure; every sum runs over the
+ * structure's rows in a fixed thread-row map and a fixed tree (no atomics, no scratch), so a structure's new state
+ * depends only on its own rows, not on its position in the batch. */
+int m3g_fire_step(const float* forces, const float* sigma, const float* energy, const int32_t* atom_ptr, int64_t B,
+                  double dt_max, double max_move, int n_min, double f_inc, double f_dec, double a_start, double f_a,
+                  double fmax_target, int max_steps, double pressure, const double* cell_factor, double* x, double* xc,
+                  double* v, double* vc, double* dt, double* a, int32_t* n_pos, int32_t* n_steps, int32_t* status,
+                  const double* L0, double* lattice, double* pos, double* fmax, double* e_frame, double* sigma_frame,
+                  void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Domain decomposition helpers (new; nothing in the reference — nn/gradient.py:26 TODO)
  * ------------------------------------------------------------------------------------------- */
 /* out[r] = in[idx[r]] rows of width W floats (halo pack) ; in[idx[r]] += add[r] (reverse halo unpack) */

@@ -1,0 +1,281 @@
+// Batched FIRE relaxation step (extension, no reference counterpart): calculator.py::Fire.step / Fire.run applied to
+// every structure of a ragged batch at once, with per-structure FIRE state, on ASE UnitCellFilter coordinates when the
+// cell relaxes.  One CTA per structure: its rows (N_b atoms, then 3 cell rows) are visited by a fixed thread-row map
+// (thread t owns rows t, t + 256, ... counted from the structure's first row) and every sum ends in the same fixed tree
+// (xor butterfly in each warp, then the 8 warp results in warp order).  The result therefore depends only on the
+// structure's own rows, never on its offset in the batch or its neighbours, and there are no atomics.
+#include "common.cuh"
+
+namespace m3g {
+
+constexpr int kFireThreads = 256;
+constexpr int kFireWarps = kFireThreads / 32;
+
+enum FireStatus { kFireRunning = 0, kFireConverged = 1, kFireNotConverged = 2, kFireFailed = 3 };
+
+struct FireArgs {
+  const float *forces, *sigma, *energy;
+  const int32_t* atom_ptr;
+  double dt_max, max_move, f_inc, f_dec, a_start, f_a, fmax_target, pressure;
+  int n_min, max_steps;
+  const double* cell_factor;
+  double *x, *xc, *v, *vc, *dt, *a;
+  int32_t *n_pos, *n_steps, *status;
+  const double* L0;
+  double *lattice, *pos, *fmax, *e_frame, *sigma_frame;
+};
+
+__device__ __forceinline__ double block_sum(double t, double* sh) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(FULL, t, o);
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
+  __syncthreads();
+  double s = 0.0;
+#pragma unroll
+  for (int q = 0; q < kFireWarps; ++q) s += sh[q];
+  __syncthreads();  // sh is reused by the next reduction
+  return s;
+}
+
+__device__ __forceinline__ double block_max(double t, double* sh) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t = fmax(t, __shfl_xor_sync(FULL, t, o));
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
+  __syncthreads();
+  double s = sh[0];
+#pragma unroll
+  for (int q = 1; q < kFireWarps; ++q) s = fmax(s, sh[q]);
+  __syncthreads();
+  return s;
+}
+
+// inverse of a row-major 3x3 matrix (adjugate / determinant)
+__device__ void inverse3(const double* m, double* inv) {
+  const double c00 = m[4] * m[8] - m[5] * m[7], c01 = m[5] * m[6] - m[3] * m[8], c02 = m[3] * m[7] - m[4] * m[6];
+  const double det = m[0] * c00 + m[1] * c01 + m[2] * c02;
+  inv[0] = c00 / det;
+  inv[1] = (m[2] * m[7] - m[1] * m[8]) / det;
+  inv[2] = (m[1] * m[5] - m[2] * m[4]) / det;
+  inv[3] = c01 / det;
+  inv[4] = (m[0] * m[8] - m[2] * m[6]) / det;
+  inv[5] = (m[2] * m[3] - m[0] * m[5]) / det;
+  inv[6] = c02 / det;
+  inv[7] = (m[1] * m[6] - m[0] * m[7]) / det;
+  inv[8] = (m[0] * m[4] - m[1] * m[3]) / det;
+}
+
+__device__ __forceinline__ double det3(const double* m) {
+  return m[0] * (m[4] * m[8] - m[5] * m[7]) + m[1] * (m[5] * m[6] - m[3] * m[8]) + m[2] * (m[3] * m[7] - m[4] * m[6]);
+}
+
+__global__ void __launch_bounds__(kFireThreads) fire_step_kernel(FireArgs p) {
+  const int64_t b = blockIdx.x;
+  if (p.status[b] != kFireRunning) return;  // finished structures stay bit-untouched
+  __shared__ double sh[kFireWarps];
+  __shared__ double D[9];      // deformation gradient D = solve(L0, L)^T, row-major
+  __shared__ double Dn[9];     // D of the updated cell rows, xc / cell_factor
+  __shared__ double cellf[9];  // generalised forces of the 3 cell rows
+  __shared__ double bc[5];     // broadcast: 1 - a, a |v|, max(|g|, 1e-30), dt, clip factor
+  __shared__ int bmode;        // 0 = stop, 1 = step with the velocity mix, 2 = step from zero velocity
+  const int64_t r0 = p.atom_ptr[b];
+  const int n = p.atom_ptr[b + 1] - p.atom_ptr[b];
+  const bool cell = p.sigma != nullptr;
+  const int tid = threadIdx.x;
+
+  if (cell && tid == 0) {
+    double L0[9], L[9], inv0[9], Dinv[9], vir[9];
+    for (int k = 0; k < 9; ++k) {
+      L0[k] = p.L0[b * 9 + k];
+      L[k] = p.lattice[b * 9 + k];
+    }
+    inverse3(L0, inv0);
+    for (int r = 0; r < 3; ++r)
+      for (int c = 0; c < 3; ++c)  // (L0^-1 L)[r][c] is D[c][r]
+        D[c * 3 + r] = inv0[r * 3 + 0] * L[0 * 3 + c] + inv0[r * 3 + 1] * L[1 * 3 + c] + inv0[r * 3 + 2] * L[2 * 3 + c];
+    const double vol = fabs(det3(L));
+    for (int k = 0; k < 9; ++k) {
+      const double s = (double)p.sigma[b * 9 + k];
+      p.sigma_frame[b * 9 + k] = s;
+      vir[k] = -vol * (k % 4 == 0 ? s + p.pressure : s);
+    }
+    inverse3(D, Dinv);
+    const double cf = p.cell_factor[b];
+    // -V (sigma + p I) D^-T / cell_factor
+    for (int r = 0; r < 3; ++r)
+      for (int c = 0; c < 3; ++c)
+        cellf[r * 3 + c] = (vir[r * 3 + 0] * Dinv[c * 3 + 0] + vir[r * 3 + 1] * Dinv[c * 3 + 1] +
+                            vir[r * 3 + 2] * Dinv[c * 3 + 2]) / cf;
+  }
+  if (tid == 0 && p.e_frame) p.e_frame[b] = (double)p.energy[b];
+  __syncthreads();
+
+  const int rows = n + (cell ? 3 : 0);
+  // generalised force of row r: F D for an atom (F itself without the cell filter), the cell force for r >= n
+  auto gen = [&](int r, double* g) {
+    if (r < n) {
+      const float* f = p.forces + (r0 + r) * 3;
+      const double f0 = f[0], f1 = f[1], f2 = f[2];
+      if (cell) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) g[c] = f0 * D[c] + f1 * D[3 + c] + f2 * D[6 + c];
+      } else {
+        g[0] = f0, g[1] = f1, g[2] = f2;
+      }
+    } else {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) g[c] = cellf[(r - n) * 3 + c];
+    }
+  };
+  auto vel = [&](int r) -> double* { return r < n ? p.v + (r0 + r) * 3 : p.vc + b * 9 + (r - n) * 3; };
+
+  // pass 1: power, |g|^2, |v|^2, max row |g|^2, finiteness
+  double P = 0.0, gg = 0.0, vv = 0.0, gmax2 = 0.0;
+  int bad = 0;
+  for (int r = tid; r < rows; r += kFireThreads) {
+    double g[3];
+    gen(r, g);
+    const double* v = vel(r);
+    const double g2 = g[0] * g[0] + g[1] * g[1] + g[2] * g[2];
+    P += g[0] * v[0] + g[1] * v[1] + g[2] * v[2];
+    gg += g2;
+    vv += v[0] * v[0] + v[1] * v[1] + v[2] * v[2];
+    gmax2 = fmax(gmax2, g2);
+    bad |= !(isfinite(g[0]) && isfinite(g[1]) && isfinite(g[2]));
+  }
+  bad = __syncthreads_or(bad);
+  P = block_sum(P, sh);
+  gg = block_sum(gg, sh);
+  vv = block_sum(vv, sh);
+  gmax2 = block_max(gmax2, sh);
+
+  if (tid == 0) {
+    const double fm = sqrt(gmax2);
+    p.fmax[b] = bad ? (double)INFINITY : fm;
+    int mode = 0;
+    if (bad) {
+      p.status[b] = kFireFailed;
+    } else if (fm < p.fmax_target) {
+      p.status[b] = kFireConverged;
+    } else if (p.n_steps[b] >= p.max_steps) {
+      p.status[b] = kFireNotConverged;
+    } else {
+      double a = p.a[b], dt = p.dt[b];
+      int n_pos = p.n_pos[b];
+      if (P > 0.0) {
+        mode = 1;
+        bc[0] = 1.0 - a;
+        bc[1] = a * sqrt(vv);
+        bc[2] = fmax(sqrt(gg), 1e-30);
+        if (n_pos > p.n_min) {
+          dt = fmin(dt * p.f_inc, p.dt_max);
+          a *= p.f_a;
+        }
+        n_pos += 1;
+      } else {
+        mode = 2;
+        a = p.a_start;
+        dt *= p.f_dec;
+        n_pos = 0;
+      }
+      p.a[b] = a;
+      p.dt[b] = dt;
+      p.n_pos[b] = n_pos;
+      p.n_steps[b] += 1;
+      bc[3] = dt;
+    }
+    bmode = mode;
+  }
+  __syncthreads();
+  const int mode = bmode;
+  if (mode == 0) return;
+  const double dt = bc[3];
+
+  // pass 2: v <- (1 - a) v + a |v| g / |g|  (or 0), v <- v + dt g; |dr|^2 with dr = dt v
+  double dr2 = 0.0;
+  for (int r = tid; r < rows; r += kFireThreads) {
+    double g[3];
+    gen(r, g);
+    double* v = vel(r);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      double w = mode == 1 ? bc[0] * v[c] + bc[1] * g[c] / bc[2] : 0.0;
+      w = w + dt * g[c];
+      v[c] = w;
+      const double d = dt * w;
+      dr2 += d * d;
+    }
+  }
+  const double norm = sqrt(block_sum(dr2, sh));
+  const bool clip = norm > p.max_move;
+  const double scale = clip ? p.max_move / norm : 1.0;
+  auto step_of = [&](double w) { const double d = dt * w; return clip ? d * scale : d; };
+
+  // pass 3: x <- x + dr, then back to Cartesian positions and lattice
+  if (!cell) {
+    for (int r = tid; r < n; r += kFireThreads) {
+      const double* v = p.v + (r0 + r) * 3;
+      double* x = p.pos + (r0 + r) * 3;
+#pragma unroll
+      for (int c = 0; c < 3; ++c) x[c] = x[c] + step_of(v[c]);
+    }
+    return;
+  }
+  if (tid < 3) {
+    const double* v = p.vc + b * 9 + tid * 3;
+    double* x = p.xc + b * 9 + tid * 3;
+    const double cf = p.cell_factor[b];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      x[c] = x[c] + step_of(v[c]);
+      Dn[tid * 3 + c] = x[c] / cf;
+    }
+  }
+  __syncthreads();
+  if (tid < 9) {  // L = L0 D^T
+    const int r = tid / 3, c = tid % 3;
+    const double* L0 = p.L0 + b * 9;
+    p.lattice[b * 9 + tid] = L0[r * 3 + 0] * Dn[c * 3 + 0] + L0[r * 3 + 1] * Dn[c * 3 + 1] + L0[r * 3 + 2] * Dn[c * 3 + 2];
+  }
+  for (int r = tid; r < n; r += kFireThreads) {
+    const double* v = p.v + (r0 + r) * 3;
+    double* x = p.x + (r0 + r) * 3;
+    double* q = p.pos + (r0 + r) * 3;
+    double xn[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) xn[c] = x[c] + step_of(v[c]);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      x[c] = xn[c];
+      q[c] = xn[0] * Dn[c * 3 + 0] + xn[1] * Dn[c * 3 + 1] + xn[2] * Dn[c * 3 + 2];
+    }
+  }
+}
+
+}  // namespace m3g
+
+using namespace m3g;
+
+extern "C" {
+
+int m3g_fire_step(const float* forces, const float* sigma, const float* energy, const int32_t* atom_ptr, int64_t B,
+                  double dt_max, double max_move, int n_min, double f_inc, double f_dec, double a_start, double f_a,
+                  double fmax_target, int max_steps, double pressure, const double* cell_factor, double* x, double* xc,
+                  double* v, double* vc, double* dt, double* a, int32_t* n_pos, int32_t* n_steps, int32_t* status,
+                  const double* L0, double* lattice, double* pos, double* fmax, double* e_frame, double* sigma_frame,
+                  void* stream) {
+  if (B == 0) return M3G_OK;
+  M3G_REQUIRE(forces && atom_ptr && v && dt && a && n_pos && n_steps && status && pos && fmax,
+              "m3g_fire_step: null pointer");
+  M3G_REQUIRE(!e_frame || energy, "m3g_fire_step: e_frame needs energy");
+  M3G_REQUIRE(!sigma || (cell_factor && x && xc && vc && L0 && lattice && sigma_frame),
+              "m3g_fire_step: the cell filter needs cell_factor, x, xc, vc, L0, lattice and sigma_frame");
+  M3G_REQUIRE(B <= 0x7fffffff, "m3g_fire_step: B=%lld too large", (long long)B);
+  FireArgs p{forces, sigma, energy, atom_ptr, dt_max, max_move, f_inc, f_dec, a_start, f_a, fmax_target, pressure,
+             n_min, max_steps, cell_factor, x, xc, v, vc, dt, a, n_pos, n_steps, status, L0, lattice, pos, fmax,
+             e_frame, sigma_frame};
+  fire_step_kernel<<<(unsigned)B, kFireThreads, 0, as_stream(stream)>>>(p);
+  M3G_LAUNCH_CHECK("m3g_fire_step");
+  return M3G_OK;
+}
+
+}  // extern "C"
