@@ -385,6 +385,15 @@ int64_t m3g_conv_tc_save_floats(int64_t E);
 int m3g_conv_tc_bwd_saved(const int32_t* src, const float* h, const float* wimgT, const float* WhT, const float* save,
                           const float* g_up, const float* g_e_base, int64_t E, int R, int mode, int passes, int n_sm,
                           float* g_e, float* g_z1, float* g_h, int gh_store, void* stream);
+/* Both adjoints of one M3GNetConv block in one launch: the node-MLP call (mode 1, g_up = g_x2, g_e_base = g_e2) and
+ * then the edge-MLP call (mode 0, g_up = g_e_base = its output ge2) of m3g_conv_tc_bwd_saved, with ge2 kept on chip.
+ * g_e, gz_node / gz_edge (nullable) and the g_h rows are bitwise those of the two calls.  gh_mode 0: the node and the
+ * edge launch's g_h rows are stored into g_h_node and g_h_edge (per-launch slices, as gh_store = 1); gh_mode 1: their
+ * sum fl(node + edge) is stored into g_h_node (g_h_edge unused, may be NULL).  g_e2 may be NULL (no residual base). */
+int m3g_conv_tc_block_bwd(const int32_t* src, const float* h, const float* n_wimgT, const float* n_WhT,
+                          const float* save_n, const float* e_wimgT, const float* e_WhT, const float* save_e,
+                          const float* g_x2, const float* g_e2, int64_t E, int R, int passes, int n_sm, float* g_e,
+                          float* gz_node, float* gz_edge, float* g_h_node, float* g_h_edge, int gh_mode, void* stream);
 
 /* adjoint of m3g_conv_tc_fwd (same outputs as m3g_conv_mlp_bwd; forward recomputed on the tensor cores).
  * wimgT = [W2d^T hi|lo, W2g^T hi|lo, W1e_dense^T hi|lo, W1e_gate^T hi|lo]: four 64x64 image pairs from
@@ -545,7 +554,7 @@ typedef struct M3GStepDesc {
   /* scratch */
   float *P, *msg;                 /* (N,512), (E,64) */
   float *g_x[2];                  /* (N,64) ping-pong; g_x[cur] holds the running adjoint */
-  float *g_e[2], *ge2;            /* (E,64) */
+  float *g_e[2], *ge2;            /* (E,64); ge2 may be NULL with fuse_conv_bwd */
   float *gz_edge, *gz_node, *gP;  /* (E,128) x 2, (N,512) */
   float *g_h, *g_hs, *g_sig_e, *g_vec4, *g_dist, *g_pos; /* (E,3), (2 n_blocks + 1, E, 3) per-launch slices, (E,9), (E,4), (E), (N,3) */
   int cur_x, cur_e;               /* state carried between phases (updated by m3g_step_run) */
@@ -554,6 +563,7 @@ typedef struct M3GStepDesc {
   int tb_split;                   /* 1: three-body forward as m3g_tb_mom_red + m3g_tb_edge_update */
   int tb_bwd_split;               /* 1: three-body backward as m3g_tb_mlp_adj (q overwrites red) + m3g_tb_mom_bwd_q */
   int fuse_e0;                    /* 1 (needs tb_split): e0 is formed inside block 0's m3g_tb_edge_update_h, never stored */
+  int fuse_conv_bwd;              /* 1: each block's node + edge MLP adjoints in one m3g_conv_tc_block_bwd (ge2 unused) */
   M3GStepBlock blocks[M3G_STEP_MAX_BLOCKS];
 } M3GStepDesc;
 

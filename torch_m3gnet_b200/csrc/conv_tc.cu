@@ -1353,6 +1353,341 @@ __global__ void __launch_bounds__(TCB2_THREADS, 1) conv_tc_bwds_kernel(ConvTcBwd
 }
 
 // --------------------------------------------------------------------------------------------------------
+// Node AND edge adjoint of one conv block in one launch: per 128-edge tile, the node MLP phase (mode 1 above) and
+// then the edge MLP phase (mode 0) on the same rows.  The node phase's output ge2 = D4 + g_e2 (dL/de2) is the edge
+// phase's upstream gradient and residual base; it is parked in the idle TMEM columns [448,512) (row-per-lane, exactly
+// the layout the edge phase reads its upstream slice in) instead of being written to and read back from HBM (768 B
+// per bond).  Per row, the MMAs and fp32 adds are those of the two conv_tc_bwds_kernel launches, in the same order, so
+// every output is bitwise identical to theirs.
+// Both MLPs' transposed images (2 x 128 KB) do not fit beside the z2 buffer and the staging tiles, so they stream
+// through a ring of two 64 KB slots (slot 0: W2d^T | W2g^T for GEMM3, slot 1: W1e_dense^T | W1e_gate^T for GEMM4),
+// refilled by cp.async.bulk from L2 as soon as the GEMM that read a slot has completed: node images, edge images, node
+// images of the next tile, ...  The z2 buffer alternates the same way (node z2 of tile t, edge z2 of t, node z2 of the
+// next tile).  Every barrier completes once per phase, so one parity bit (flipped per phase) serves all of them.
+struct ConvTcBlockBwdParams {
+  const int32_t* src; const float* h;
+  const float* wimgT[2];  // [node, edge], each as ConvTcBwdSParams::wimgT
+  const float* WhT[2]; const float* save[2];
+  const float* g_x2; const float* g_e2;
+  int64_t E; int R; int passes;
+  float* g_e; float* g_z1[2]; float* g_h[2];
+  int gh_mode;  // 0: node / edge g_h rows stored into g_h[0] / g_h[1]; 1: fl(node + edge) stored into g_h[0]
+};
+constexpr int SMEM_RING_SLOT = 2 * SMEM_S_BYTES;                   // 65536: the image pairs of one GEMM pair
+constexpr int SMEM_BB_MISC = 2 * TC_BWD_MAX_R * 64 * 4 + 64;  // Wh^T of both MLPs, 5 mbarriers, TMEM slot, image pointers
+constexpr int SMEM_BLOCK_BWD_BYTES = 2 * SMEM_RING_SLOT + 16 * STG_WARP_BYTES + SMEM_Z2_BYTES + SMEM_BB_MISC + 1024;
+static_assert(SMEM_BLOCK_BWD_BYTES <= 232448, "fused block backward exceeds the 227 KB shared-memory limit");
+
+__global__ void __launch_bounds__(TCB2_THREADS, 1) conv_tc_block_bwd_kernel(ConvTcBlockBwdParams p) {
+  extern __shared__ __align__(1024) char smem_raw[];
+  char* smem = (char*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
+  const uint32_t sbase = smem_u32(smem);
+  const uint32_t ring0 = sbase, ring1 = sbase + SMEM_RING_SLOT;
+  const uint32_t stg_all = sbase + 2 * SMEM_RING_SLOT;
+  const uint32_t z2buf = stg_all + 16 * STG_WARP_BYTES;
+  float* misc = reinterpret_cast<float*>(smem + 2 * SMEM_RING_SLOT + 16 * STG_WARP_BYTES + SMEM_Z2_BYTES);
+  const uint32_t wh_a = z2buf + SMEM_Z2_BYTES;  // [node | edge] Wh^T
+  uint64_t* bars = reinterpret_cast<uint64_t*>(misc + 2 * TC_BWD_MAX_R * 64);
+  uint32_t* tmem_slot_p = reinterpret_cast<uint32_t*>(bars + 5);
+  // [node, edge] image addresses, re-read from shared memory by the refilling thread: as loop invariants held in
+  // registers they would be spilled
+  const float** wsrc = reinterpret_cast<const float**>(bars + 6);
+  auto image_src = [&](int m) {
+    uint64_t a;
+    asm volatile("ld.shared.u64 %0, [%1];" : "=l"(a) : "r"(smem_u32(wsrc + m)));
+    return reinterpret_cast<const float*>(a);
+  };
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int q = warp & 3, cs = warp >> 2;
+  const int row = 32 * q + lane;
+  const int k0 = 16 * cs;
+  const uint32_t stg = stg_all + warp * STG_WARP_BYTES;
+  const int cr = lane >> 2, cc4 = lane & 3;
+  const int R = p.R;
+  constexpr uint32_t HALF_IMG_FLOATS = SMEM_RING_SLOT / 4;
+
+  for (int i = tid; i < 2 * TC_BWD_MAX_R * 64; i += TCB2_THREADS) {
+    const int j = i % (TC_BWD_MAX_R * 64);
+    misc[i] = (j < R * 64) ? p.WhT[i / (TC_BWD_MAX_R * 64)][j] : 0.0f;
+  }
+  if (warp == 0) tmem_alloc<512>(tmem_slot_p);
+  if (tid == 0) {
+#pragma unroll
+    for (int i = 0; i < 5; ++i) mbar_init(&bars[i], 1);
+    mbar_fence_init();
+  }
+  fence_proxy_async();
+  fence_before_sync();
+  __syncthreads();
+  fence_after_sync();
+  if (*tmem_slot_p != 0u) __trap();  // one CTA per SM owns all 512 columns: literal operand addresses (see bwd2)
+  constexpr uint32_t tmem = 0u;
+  const uint32_t t_lane = ((uint32_t)(32 * q) << 16);
+  constexpr uint32_t AH = 0, AL = 64, A2H = 128, A2L = 192, D3D = 256, D3G = 320, D4 = 384, GE2 = 448;
+  uint64_t *bar3 = &bars[0], *bar4 = &bars[1], *zb = &bars[2], *rb0 = &bars[3], *rb1 = &bars[4];
+
+  const int n_tiles = (int)((p.E + TILE_M - 1) / TILE_M);
+  if (tid == 0 && (int)blockIdx.x < n_tiles) {
+    wsrc[0] = p.wimgT[0];
+    wsrc[1] = p.wimgT[1];
+    const float* w = image_src(0);
+    mbar_arrive_expect_tx(rb0, SMEM_RING_SLOT);
+    bulk_g2s(ring0, w, SMEM_RING_SLOT, rb0);
+    mbar_arrive_expect_tx(rb1, SMEM_RING_SLOT);
+    bulk_g2s(ring1, w + HALF_IMG_FLOATS, SMEM_RING_SLOT, rb1);
+    mbar_arrive_expect_tx(zb, SMEM_Z2_BYTES);
+    bulk_g2s(z2buf, p.save[0] + save_offset(blockIdx.x, 2, 0, 0), SMEM_Z2_BYTES, zb);
+  }
+  uint32_t par = 0;
+  // the node phase's upstream slice g_x2[src] of the next tile is requested one tile ahead (see conv_tc_bwds_kernel)
+  float4 gnext[4];
+  auto load_upstream = [&](int s_atom) {
+    const float* gr = p.g_x2 + (int64_t)s_atom * TC_F + k0;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) gnext[c] = __ldg(reinterpret_cast<const float4*>(gr + 4 * c));
+  };
+  if ((int)blockIdx.x < n_tiles) load_upstream(__ldg(p.src + min((int64_t)blockIdx.x * TILE_M + row, p.E - 1)));
+  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int64_t e0 = (int64_t)tile * TILE_M;
+    const int eg = (int)min(e0 + row, p.E - 1);  // E * R < 2^31 (checked by the host entry)
+    const bool live = (e0 + row) < p.E;
+    const bool more = tile + (int)gridDim.x < n_tiles;
+    const int64_t ebase = e0 + 32 * q + cr;
+#pragma unroll
+    for (int m = 0; m < 2; ++m) {  // m = 0: node MLP (upstream g_x2[src]), m = 1: edge MLP (upstream ge2)
+      const bool node = m == 0;
+      const bool next_phase = node || more;
+      {
+        // next phase's SiLU'(z1) blocks into L2 (its z2 blocks arrive by bulk copy); the node phase also pulls the
+        // next tile's g_e2 rows and h
+        const int tn = node ? tile : tile + (int)gridDim.x;
+        if (tn < n_tiles) prefetch_l2(p.save[m ^ 1] + (int64_t)tn * SAVE_TILE_WORDS + tid * 32);
+        if (node && more) {
+          const int64_t en = (int64_t)(tile + gridDim.x) * TILE_M;
+          const int64_t rn = min(en + (tid & 255) / 2, p.E - 1);
+          if (tid < 256) {
+            if (p.g_e2) prefetch_l2(p.g_e2 + rn * TC_F + (tid & 1) * 32);
+          } else if (tid < 256 + 16) {
+            prefetch_l2(p.h + min(en * R + (tid - 256) * 32, p.E * R - 1));
+          }
+        }
+      }
+      // ---- T0: upstream gradient slice, saved z2 slices, h ----
+      float zd[16], zg[16], gu[16];
+      if (node) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          gu[4 * c] = gnext[c].x; gu[4 * c + 1] = gnext[c].y; gu[4 * c + 2] = gnext[c].z; gu[4 * c + 3] = gnext[c].w;
+        }
+      } else {
+        tmem_ld16(t_lane + GE2 + k0, gu);  // written by this thread in the node phase
+        tmem_ld_wait();
+      }
+      {
+        mbar_wait_warp(zb, par);
+        const uint32_t s2 = z2buf + ((cs * 4 + q) << 11) + 16 * lane;
+        const uint32_t s3 = s2 + (16 << 11);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          float4 a = lds128(s2 + 512 * c);
+          float4 b = lds128(s3 + 512 * c);
+          zd[4 * c] = a.x; zd[4 * c + 1] = a.y; zd[4 * c + 2] = a.z; zd[4 * c + 3] = a.w;
+          zg[4 * c] = b.x; zg[4 * c + 1] = b.y; zg[4 * c + 2] = b.z; zg[4 * c + 3] = b.w;
+        }
+      }
+      float hm[TC_BWD_MAX_R], ghp[TC_BWD_MAX_R];
+#pragma unroll
+      for (int mm = 0; mm < TC_BWD_MAX_R; ++mm) {
+        hm[mm] = (mm < R) ? __ldg(p.h + eg * R + mm) : 0.0f;
+        ghp[mm] = 0.0f;
+      }
+      // ---- T5: output-stage adjoint -> dz2d (operand A), dz2g (operand A2) ; GEMM3d + GEMM3g ----
+      const uint32_t whm = wh_a + m * (TC_BWD_MAX_R * 64 * 4);
+#pragma unroll
+      for (int c = 0; c < 16; c += 4) {
+        float whv[TC_BWD_MAX_R][4];
+#pragma unroll
+        for (int mm = 0; mm < TC_BWD_MAX_R; ++mm) {
+          float4 w4 = lds128(whm + 4 * (mm * 64 + k0 + c));
+          whv[mm][0] = w4.x; whv[mm][1] = w4.y; whv[mm][2] = w4.z; whv[mm][3] = w4.w;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const float z = zd[c + u];
+          const float sgm = sigmoid_fast(z);
+          const float sd = z * sgm;
+          const float sgr = sgm * (1.0f + z * (1.0f - sgm));
+          const float sg = sigmoid_fast(zg[c + u]);
+          float s = 0.0f;
+#pragma unroll
+          for (int mm = 0; mm < TC_BWD_MAX_R; ++mm) s += hm[mm] * whv[mm][u];
+          const float gs = gu[c + u] * sd * sg;
+#pragma unroll
+          for (int mm = 0; mm < TC_BWD_MAX_R; ++mm) ghp[mm] += gs * whv[mm][u];
+          const float gphi = gu[c + u] * s;
+          zd[c + u] = gphi * sg * sgr;               // dz2d
+          zg[c + u] = gphi * sd * sg * (1.0f - sg);  // dz2g
+        }
+      }
+      tmem_put_split16(t_lane + AH + k0, t_lane + AL + k0, zd);
+      tmem_put_split16(t_lane + A2H + k0, t_lane + A2L + k0, zg);
+      if (cs != 0) sts128(stg + lane * 16, make_float4(ghp[0], ghp[1], ghp[2], 0.0f));
+      tmem_st_wait();
+      fence_before_sync();
+      __syncthreads();
+      if (tid == 0) {
+        fence_after_sync();
+        if (next_phase) {  // every thread has consumed this phase's z2: refill for the next phase
+          fence_proxy_async();
+          mbar_arrive_expect_tx(zb, SMEM_Z2_BYTES);
+          bulk_g2s(z2buf, p.save[m ^ 1] + save_offset(node ? tile : tile + (int)gridDim.x, 2, 0, 0), SMEM_Z2_BYTES, zb);
+        }
+        mbar_wait(rb0, par);
+        issue_gemm_ts(tmem + D3D, tmem + AH, tmem + AL, ring0, ring0 + IMG_W2 * 4, 64, 64, false, p.passes);
+        issue_gemm_ts(tmem + D3G, tmem + A2H, tmem + A2L, ring0 + SMEM_S_BYTES, ring0 + SMEM_S_BYTES + IMG_W2 * 4, 64,
+                      64, false, p.passes);
+        commit(bar3);
+      }
+      if (cs == 0) {
+        float4 g1 = lds128(stg + 4 * STG_WARP_BYTES + lane * 16);
+        float4 g2 = lds128(stg + 8 * STG_WARP_BYTES + lane * 16);
+        float4 g3 = lds128(stg + 12 * STG_WARP_BYTES + lane * 16);
+        if (live) {
+          float tot[3] = {((ghp[0] + g1.x) + g2.x) + g3.x, ((ghp[1] + g1.y) + g2.y) + g3.y,
+                          ((ghp[2] + g1.z) + g2.z) + g3.z};
+          float* gh = p.g_h[p.gh_mode ? 0 : m];
+          if (p.gh_mode && !node) {  // this thread stored the node rows in this tile's node phase
+#pragma unroll
+            for (int mm = 0; mm < TC_BWD_MAX_R; ++mm)
+              if (mm < R) gh[eg * R + mm] += tot[mm];
+          } else {
+#pragma unroll
+            for (int mm = 0; mm < TC_BWD_MAX_R; ++mm)
+              if (mm < R) gh[eg * R + mm] = tot[mm];
+          }
+        }
+      }
+      // saved SiLU'(z1) slices (dense -> zd, gate -> zg), in flight while GEMM3 runs
+      int s_next = 0;  // edge phase: source atom of this row in the next tile
+      if (!node && more) s_next = __ldg(p.src + min((int64_t)(tile + gridDim.x) * TILE_M + row, p.E - 1));
+      {
+        const float* s0 = p.save[m] + save_offset(tile, 0, cs, q) + 4 * lane;
+        const float* s1 = p.save[m] + save_offset(tile, 1, cs, q) + 4 * lane;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          float4 a = __ldg(reinterpret_cast<const float4*>(s0 + 128 * c));
+          float4 b = __ldg(reinterpret_cast<const float4*>(s1 + 128 * c));
+          zd[4 * c] = a.x; zd[4 * c + 1] = a.y; zd[4 * c + 2] = a.z; zd[4 * c + 3] = a.w;
+          zg[4 * c] = b.x; zg[4 * c + 1] = b.y; zg[4 * c + 2] = b.z; zg[4 * c + 3] = b.w;
+        }
+      }
+      // ---- T6: dz1 = D3 * SiLU'(z1) -> operands A (dense), A2 (gate) ; GEMM4a + GEMM4b ----
+      mbar_wait_warp(bar3, par);
+      fence_after_sync();
+      if (tid == 0 && next_phase) {  // GEMM3 has read slot 0: the next phase's GEMM3 images
+        mbar_arrive_expect_tx(rb0, SMEM_RING_SLOT);
+        bulk_g2s(ring0, image_src(m ^ 1), SMEM_RING_SLOT, rb0);
+      }
+      {
+        float v[16];
+        tmem_ld16(t_lane + D3D + k0, v);
+        tmem_ld_wait();
+#pragma unroll
+        for (int c = 0; c < 16; ++c) zd[c] *= v[c];
+        tmem_put_split16(t_lane + AH + k0, t_lane + AL + k0, zd);
+        tmem_ld16(t_lane + D3G + k0, v);
+        tmem_ld_wait();
+#pragma unroll
+        for (int c = 0; c < 16; ++c) zg[c] *= v[c];
+        tmem_put_split16(t_lane + A2H + k0, t_lane + A2L + k0, zg);
+      }
+      tmem_st_wait();
+      fence_before_sync();
+      __syncthreads();
+      if (tid == 0) {
+        fence_after_sync();
+        mbar_wait(rb1, par);
+        issue_gemm_ts(tmem + D4, tmem + AH, tmem + AL, ring1, ring1 + IMG_W2 * 4, 64, 64, false, p.passes);
+        issue_gemm_ts(tmem + D4, tmem + A2H, tmem + A2L, ring1 + SMEM_S_BYTES, ring1 + SMEM_S_BYTES + IMG_W2 * 4, 64,
+                      64, true, p.passes);
+        commit(bar4);
+      }
+      float4 gb[4];
+      if (node && p.g_e2) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+          gb[i] = __ldg(reinterpret_cast<const float4*>(p.g_e2 + min(ebase + 8 * i, p.E - 1) * TC_F + k0 + 4 * cc4));
+      }
+      float* gz = p.g_z1[m];
+      if (gz != nullptr) {
+#pragma unroll
+        for (int hb = 0; hb < 2; ++hb) {
+          const float* dz = hb ? zg : zd;
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            sts128(stg + stg_off(lane, c), make_float4(dz[4 * c], dz[4 * c + 1], dz[4 * c + 2], dz[4 * c + 3]));
+          __syncwarp();
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            float4 r4 = lds128(stg + stg_off(8 * i + cr, cc4));
+            if (ebase + 8 * i < p.E) *reinterpret_cast<float4*>(gz + (ebase + 8 * i) * 128 + 64 * hb + k0 + 4 * cc4) = r4;
+          }
+          __syncwarp();
+        }
+      }
+      if (!node && more) load_upstream(s_next);
+      // ---- T7: ge2 = D4 + g_e2 into TMEM (node) | g_e = D4 + ge2 (edge) ----
+      mbar_wait_warp(bar4, par);
+      fence_after_sync();
+      if (tid == 0 && next_phase) {  // GEMM4 has read slot 1: the next phase's GEMM4 images
+        mbar_arrive_expect_tx(rb1, SMEM_RING_SLOT);
+        bulk_g2s(ring1, image_src(m ^ 1) + HALF_IMG_FLOATS, SMEM_RING_SLOT, rb1);
+      }
+      if (node) {
+        float v[16];
+        tmem_ld16(t_lane + D4 + k0, v);
+        tmem_ld_wait();
+        if (p.g_e2) {
+#pragma unroll
+          for (int i = 0; i < 4; ++i) sts128(stg + stg_off(8 * i + cr, cc4), gb[i]);
+          __syncwarp();
+#pragma unroll
+          for (int c = 0; c < 4; ++c) {
+            float4 b = lds128(stg + stg_off(lane, c));
+            v[4 * c] += b.x; v[4 * c + 1] += b.y; v[4 * c + 2] += b.z; v[4 * c + 3] += b.w;
+          }
+          __syncwarp();
+        }
+        tmem_st16(t_lane + GE2 + k0, v);
+        tmem_st_wait();
+      } else {
+        float v[16], b[16];
+        tmem_ld16(t_lane + D4 + k0, v);
+        tmem_ld16(t_lane + GE2 + k0, b);
+        tmem_ld_wait();
+#pragma unroll
+        for (int c = 0; c < 4; ++c)
+          sts128(stg + stg_off(lane, c), make_float4(v[4 * c] + b[4 * c], v[4 * c + 1] + b[4 * c + 1],
+                                                     v[4 * c + 2] + b[4 * c + 2], v[4 * c + 3] + b[4 * c + 3]));
+        __syncwarp();
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          float4 r4 = lds128(stg + stg_off(8 * i + cr, cc4));
+          if (ebase + 8 * i < p.E) *reinterpret_cast<float4*>(p.g_e + (ebase + 8 * i) * TC_F + k0 + 4 * cc4) = r4;
+        }
+        __syncwarp();
+      }
+      fence_before_sync();
+      par ^= 1;
+    }
+  }
+  fence_before_sync();
+  __syncthreads();
+  if (warp == 0) tmem_dealloc<512>(tmem);
+}
+
+// --------------------------------------------------------------------------------------------------------
 // debug: issue rate of tcgen05.mma kind::tf32 M=128 for a given N, A from shared (0) or tensor memory (1)
 template <int N, int ATMEM>
 __global__ void __launch_bounds__(128, 1) mma_rate_kernel(int n_rep, long long* out) {
@@ -1589,6 +1924,33 @@ int m3g_conv_tc_bwd_saved(const int32_t* src, const float* h, const float* wimgT
   unsigned grid = (unsigned)((n_tiles < n_sm) ? n_tiles : n_sm);
   conv_tc_bwds_kernel<<<grid, TCB2_THREADS, SMEM_BWDS_BYTES, as_stream(stream)>>>(p);
   M3G_LAUNCH_CHECK("m3g_conv_tc_bwd_saved");
+  return M3G_OK;
+}
+
+int m3g_conv_tc_block_bwd(const int32_t* src, const float* h, const float* n_wimgT, const float* n_WhT,
+                          const float* save_n, const float* e_wimgT, const float* e_WhT, const float* save_e,
+                          const float* g_x2, const float* g_e2, int64_t E, int R, int passes, int n_sm, float* g_e,
+                          float* gz_node, float* gz_edge, float* g_h_node, float* g_h_edge, int gh_mode, void* stream) {
+  if (E == 0) return M3G_OK;
+  M3G_REQUIRE(gh_mode == 0 || gh_mode == 1, "m3g_conv_tc_block_bwd: gh_mode must be 0 or 1");
+  M3G_REQUIRE(src && h && n_wimgT && n_WhT && save_n && e_wimgT && e_WhT && save_e && g_x2 && g_e && g_h_node &&
+                  (gh_mode == 1 || g_h_edge),
+              "m3g_conv_tc_block_bwd: null pointer");
+  M3G_REQUIRE(R >= 1 && R <= TC_BWD_MAX_R, "m3g_conv_tc_block_bwd: R=%d unsupported (max %d)", R, TC_BWD_MAX_R);
+  M3G_REQUIRE(E * R < ((int64_t)1 << 31), "m3g_conv_tc_block_bwd: E * R must be below 2^31");
+  M3G_REQUIRE(passes == 1 || passes == 3, "m3g_conv_tc_block_bwd: passes must be 1 or 3");
+  cudaError_t err =
+      cudaFuncSetAttribute(conv_tc_block_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BLOCK_BWD_BYTES);
+  if (err != cudaSuccess) {
+    set_error("m3g_conv_tc_block_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(err));
+    return M3G_ERR_CUDA;
+  }
+  ConvTcBlockBwdParams p{src, h, {n_wimgT, e_wimgT}, {n_WhT, e_WhT}, {save_n, save_e}, g_x2, g_e2, E, R, passes,
+                         g_e, {gz_node, gz_edge}, {g_h_node, g_h_edge}, gh_mode};
+  int64_t n_tiles = (E + TILE_M - 1) / TILE_M;
+  unsigned grid = (unsigned)((n_tiles < n_sm) ? n_tiles : n_sm);
+  conv_tc_block_bwd_kernel<<<grid, TCB2_THREADS, SMEM_BLOCK_BWD_BYTES, as_stream(stream)>>>(p);
+  M3G_LAUNCH_CHECK("m3g_conv_tc_block_bwd");
   return M3G_OK;
 }
 

@@ -90,10 +90,16 @@ int conv_bwd(M3GStepDesc* d, int b, void* s) {
   // every backward launch stores its radial-weight adjoint into its own slice; the epilogue sums the slices
   float* gh_node = d->g_hs + (int64_t)(2 * (d->n_blocks - 1 - b)) * R * d->E;
   float* gh_edge = gh_node + (int64_t)R * d->E;
-  M3G_TRY(m3g_conv_tc_bwd_saved(d->src, d->h, k.n_wimgT, k.n_WhT, k.save_n, g_x2, g_e2, d->E, R, 1, d->passes, d->n_sm,
-                                d->ge2, need_x ? d->gz_node : nullptr, gh_node, 1, s));
-  M3G_TRY(m3g_conv_tc_bwd_saved(d->src, d->h, k.e_wimgT, k.e_WhT, k.save_e, d->ge2, d->ge2, d->E, R, 0, d->passes,
-                                d->n_sm, g_e_new, need_x ? d->gz_edge : nullptr, gh_edge, 1, s));
+  if (d->fuse_conv_bwd) {
+    M3G_TRY(m3g_conv_tc_block_bwd(d->src, d->h, k.n_wimgT, k.n_WhT, k.save_n, k.e_wimgT, k.e_WhT, k.save_e, g_x2, g_e2,
+                                  d->E, R, d->passes, d->n_sm, g_e_new, need_x ? d->gz_node : nullptr,
+                                  need_x ? d->gz_edge : nullptr, gh_node, gh_edge, 0, s));
+  } else {
+    M3G_TRY(m3g_conv_tc_bwd_saved(d->src, d->h, k.n_wimgT, k.n_WhT, k.save_n, g_x2, g_e2, d->E, R, 1, d->passes,
+                                  d->n_sm, d->ge2, need_x ? d->gz_node : nullptr, gh_node, 1, s));
+    M3G_TRY(m3g_conv_tc_bwd_saved(d->src, d->h, k.e_wimgT, k.e_WhT, k.save_e, d->ge2, d->ge2, d->E, R, 0, d->passes,
+                                  d->n_sm, g_e_new, need_x ? d->gz_edge : nullptr, gh_edge, 1, s));
+  }
   d->cur_e = d->have_g_e ? (d->cur_e ^ 1) : 0;
   d->have_g_e = 1;
   if (need_x) {

@@ -55,7 +55,7 @@ class _Desc(ctypes.Structure):
                 + [(n, _fp) for n in ("ge2", "gz_edge", "gz_node", "gP", "g_h", "g_hs", "g_sig_e", "g_vec4", "g_dist",
                                       "g_pos")]
                 + [(n, ctypes.c_int) for n in ("cur_x", "cur_e", "have_g_e", "msg_reduce", "tb_split",
-                                               "tb_bwd_split", "fuse_e0")]
+                                               "tb_bwd_split", "fuse_e0", "fuse_conv_bwd")]
                 + [("blocks", _Block * MAX_BLOCKS)])
 
 
@@ -179,11 +179,14 @@ class StepEngine:
             K.FORCES: torch.empty((N, 3), **f32), K.STRESSES: torch.empty((B, 6), **f32),
         }
         n_save = int(_lib.LIB.load().m3g_conv_tc_save_floats(E))
+        fuse_bwd = bool(conv_mod.CONV_BWD_FUSED)
         # scratch: one allocation carved by offsets (floats, every piece 16-byte aligned)
         sizes: List = [("vec4", 4 * E), ("x0", 64 * N), ("e0", 64 * E), ("P", 512 * N), ("msg", 64 * E),
-                       ("g_x0", 64 * N), ("g_x1", 64 * N), ("g_e0", 64 * E), ("g_e1", 64 * E), ("ge2", 64 * E),
-                       ("gz_edge", 128 * E), ("gz_node", 128 * E), ("gP", 512 * N), ("g_h", 3 * E), ("g_hs", (2 * n + 1) * 3 * E),
+                       ("g_x0", 64 * N), ("g_x1", 64 * N), ("g_e0", 64 * E), ("g_e1", 64 * E), ("gz_edge", 128 * E),
+                       ("gz_node", 128 * E), ("gP", 512 * N), ("g_h", 3 * E), ("g_hs", (2 * n + 1) * 3 * E),
                        ("g_sig_e", 9 * E), ("g_vec4", 4 * E), ("g_dist", E), ("g_pos", 3 * N)]
+        if not fuse_bwd:  # the fused block backward keeps ge2 on chip
+            sizes.append(("ge2", 64 * E))
         tables: Dict = {}
         weights = []
         for b in range(n):
@@ -214,6 +217,7 @@ class StepEngine:
         d.tb_split = int(interaction.TB_SPLIT)
         d.tb_bwd_split = int(interaction.TB_BWD_SPLIT)
         d.fuse_e0 = int(interaction.TB_SPLIT and FUSE_E0)
+        d.fuse_conv_bwd = int(fuse_bwd)
         d.n_members = int(plan.n_members)
         d.length_scale, d.energy_scale = float(self.scale.length_scale), float(self.readout.scale)
         d.r3 = float(weights[0][0]["r3"])
@@ -246,9 +250,10 @@ class StepEngine:
         d.atomic, d.scaled_total, d.total = (_p(out[K.SCALED_ATOMIC_ENERGIES]), _p(out[K.SCALED_TOTAL_ENERGY]),
                                              _p(out[K.TOTAL_ENERGY]))
         d.forces, d.stresses = _p(out[K.FORCES]), _p(out[K.STRESSES])
-        for name in ("vec4", "x0", "e0", "P", "msg", "ge2", "gz_edge", "gz_node", "gP", "g_h", "g_hs", "g_sig_e",
-                     "g_vec4", "g_dist", "g_pos"):
+        for name in ("vec4", "x0", "e0", "P", "msg", "gz_edge", "gz_node", "gP", "g_h", "g_hs", "g_sig_e", "g_vec4",
+                     "g_dist", "g_pos"):
             setattr(d, name, at(name))
+        d.ge2 = None if fuse_bwd else at("ge2")
         d.g_x[0], d.g_x[1] = at("g_x0"), at("g_x1")
         d.g_e[0], d.g_e[1] = at("g_e0"), at("g_e1")
         x_final, e_final = out[K.NODE_FEATURES].data_ptr(), out[K.EDGE_ATTR].data_ptr()
@@ -289,14 +294,17 @@ class StepEngine:
     def launches(self, with_angles: bool = True, stress: bool = False) -> int:
         """Kernel launches of one full step (for bench.py's gpu_launches): prologue 7 (6 when e0 is formed inside the first three-body edge update; +1 for the cos output) + one
         radial table per distinct constant set, 6 per block forward, 2 for the readout with its adjoint, 7 per block
-        backward (3 for block 0, whose node-feature gradient is dead; +1 per block with the split three-body adjoint), 4 in the epilogue, 2 for forces + virial;
-        +2 for the cell stress (m3g_bond_virial) when ``stress`` is set."""
+        backward (3 for block 0, whose node-feature gradient is dead; one less per block when the node and edge MLP
+        adjoints run as one launch; +1 per block with the split three-body adjoint), 4 in the epilogue, 2 for forces +
+        virial; +2 for the cell stress (m3g_bond_virial) when ``stress`` is set."""
         n = self.n_blocks
         tables = len({t._packed.get()["consts_key"] for t in self.tbs})
+        from torch_m3gnet_b200.nn import conv as conv_mod
         from torch_m3gnet_b200.nn import interaction
 
         return (7 - int(interaction.TB_SPLIT and FUSE_E0) + int(with_angles) + tables + (6 + int(interaction.TB_SPLIT)) * n + 2
-                + (7 * n - 4 + int(interaction.TB_BWD_SPLIT) * n) + 4 + 2 + 2 * int(stress))
+                + ((7 - int(conv_mod.CONV_BWD_FUSED)) * n - 4 + int(interaction.TB_BWD_SPLIT) * n) + 4 + 2
+                + 2 * int(stress))
 
     @staticmethod
     def cell_stress(keep) -> torch.Tensor:

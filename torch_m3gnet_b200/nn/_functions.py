@@ -43,6 +43,12 @@ def msg_reduce() -> bool:
     return conv.MSG_REDUCE
 
 
+def conv_bwd_fused() -> bool:
+    from torch_m3gnet_b200.nn import conv
+
+    return conv.CONV_BWD_FUSED
+
+
 def conv_path() -> str:
     from torch_m3gnet_b200.nn import conv
 
@@ -342,7 +348,6 @@ class ConvFn(Function):
         g_x2, g_e2 = g_x2.contiguous(), _c(g_e2)
         g_h = torch.zeros_like(h)
         nd, ed = w["node"], w["edge"]
-        ge2 = torch.empty_like(e)
         gz_node = _empty((E, 2 * F), x)
         g_e = torch.empty_like(e)
         gz_edge = _empty((E, 2 * F), x)
@@ -351,13 +356,20 @@ class ConvFn(Function):
         if save_e is not None:
             passes = 3 if path == "tc3" else 1
             n_sm = sm_count(x.device)
-            # g_h: the node launch stores its rows, the edge launch adds to them (no zero fill needed)
-            call("conv_tc_bwd_saved", plan.src, h, nd["wimgT"], nd["WhT"], save_n, g_x2, g_e2, E, R, 1, passes, n_sm, ge2,
-                 gz_node, g_h, 1)
-            call("conv_tc_bwd_saved", plan.src, h, ed["wimgT"], ed["WhT"], save_e, ge2, ge2, E, R, 0, passes, n_sm, g_e,
-                 gz_edge, g_h, 0)
+            if conv_bwd_fused():
+                # g_h = fl(node + edge) rows, as the two launches below leave them
+                call("conv_tc_block_bwd", plan.src, h, nd["wimgT"], nd["WhT"], save_n, ed["wimgT"], ed["WhT"], save_e,
+                     g_x2, g_e2, E, R, passes, n_sm, g_e, gz_node, gz_edge, g_h, None, 1)
+            else:
+                ge2 = torch.empty_like(e)
+                # g_h: the node launch stores its rows, the edge launch adds to them (no zero fill needed)
+                call("conv_tc_bwd_saved", plan.src, h, nd["wimgT"], nd["WhT"], save_n, g_x2, g_e2, E, R, 1, passes, n_sm,
+                     ge2, gz_node, g_h, 1)
+                call("conv_tc_bwd_saved", plan.src, h, ed["wimgT"], ed["WhT"], save_e, ge2, ge2, E, R, 0, passes, n_sm,
+                     g_e, gz_edge, g_h, 0)
             ctx.saved_acts = (None, None)
         elif F == 64 and "wimgT" in ed and path in ("tc3", "tc1") and R <= 3:
+            ge2 = torch.empty_like(e)
             passes = 3 if path == "tc3" else 1
             n_sm = sm_count(x.device)
             call("conv_tc_bwd", P, 8 * F, 4 * F, plan.src, plan.dst, e2, h, nd["wimg"], nd["wimgT"], nd["b2d"], nd["b2g"],
@@ -365,6 +377,7 @@ class ConvFn(Function):
             call("conv_tc_bwd", P, 8 * F, 0, plan.src, plan.dst, e, h, ed["wimg"], ed["wimgT"], ed["b2d"], ed["b2g"],
                  ed["WhT"], ge2, ge2, E, R, 0, passes, n_sm, g_e, gz_edge, g_h)
         else:
+            ge2 = torch.empty_like(e)
             call("conv_mlp_bwd", P, 8 * F, 4 * F, plan.src, plan.dst, e2, h, nd["W1eT"], nd["W2dT"], nd["b2d"],
                  nd["W2gT"], nd["b2g"], nd["WhT"], nd["W1e"], nd["W2d"], nd["W2g"], nd["Wh"], g_x2, g_e2, E, F, R, 1,
                  ge2, gz_node, g_h)

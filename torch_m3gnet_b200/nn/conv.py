@@ -22,6 +22,10 @@ TC_BWD_VARIANT = int(os.environ.get("M3G_TC_BWD_VARIANT", "4"))
 # of the sum then follows the 32-row blocks of the batch's bond list, so the same structure in another batch position
 # agrees to fp32 rounding instead of bit for bit.  False: messages written row by row and summed in ascending bond order.
 MSG_REDUCE = os.environ.get("M3G_CONV_MSG_REDUCE", "1") != "0"
+# True (default): the backward from saved activations runs the node and the edge MLP adjoint of a block in one launch
+# (m3g_conv_tc_block_bwd), keeping dL/de2 on chip instead of a 256 B / bond write and two reads; bitwise the same
+# results.  False: two m3g_conv_tc_bwd_saved launches.
+CONV_BWD_FUSED = os.environ.get("M3G_CONV_BWD_FUSED", "1") != "0"
 
 
 def _tc_images(w1e: torch.Tensor, w2d: torch.Tensor, w2g: torch.Tensor) -> torch.Tensor:
