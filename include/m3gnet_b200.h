@@ -65,7 +65,7 @@ int m3g_csr_by_key(const int32_t* keys, int64_t n, int64_t n_rows, int32_t* row_
 int m3g_gather_i32(const int32_t* vals, const int32_t* perm, int64_t n, int32_t* out, void* stream);
 /* every row of (row_ptr, cols) is sorted ascending in place (rows are short: one neighbour shell) */
 int m3g_sort_rows(const int32_t* row_ptr, int64_t n_rows, int32_t* cols, void* stream);
-/* flags[0] = 1 iff (ptr_a, col_a) == transpose(ptr_a, col_a), i.e. (e1,e2) present <=> (e2,e1) present */
+/* flags[0] = 1 iff (ptr_a, col_a) == transpose(ptr_a, col_a), i.e. (e1,e2) occurs as often as (e2,e1); rows sorted */
 int m3g_csr_is_symmetric(const int32_t* row_ptr, const int32_t* cols, int64_t n_rows, int32_t* flags,
                          void* stream);
 

@@ -181,23 +181,29 @@ __global__ void gather_i32_kernel(const int32_t* __restrict__ vals, const int32_
   if (i < n) out[i] = vals[perm[i]];
 }
 
-// symmetric iff for every (r, c) there is (c, r): binary search in row c (rows sorted ascending)
+// symmetric iff for every (r, c) the pair (c, r) occurs as often as (r, c): the transpose is then the matrix itself,
+// repeated entries included (a repeated triplet is summed once per occurrence, so the transpose must repeat it too).
+// Rows sorted ascending: each run of c in row r is compared with the run of r in row c (two binary searches).
 __global__ void csr_symmetric_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ cols,
                                      int64_t n_rows, int32_t* __restrict__ flags) {
   int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n_rows) return;
-  for (int32_t p = row_ptr[r]; p < row_ptr[r + 1]; ++p) {
-    int32_t c = cols[p];
+  const int32_t end = row_ptr[r + 1];
+  for (int32_t p = row_ptr[r]; p < end;) {
+    const int32_t c = cols[p];
     if (c < 0 || c >= n_rows) { flags[0] = 0; return; }
+    int32_t q = p + 1;
+    while (q < end && cols[q] == c) ++q;
     int32_t lo = row_ptr[c], hi = row_ptr[c + 1];
-    bool found = false;
-    while (lo < hi) {
-      int32_t mid = (lo + hi) >> 1;
-      int32_t v = cols[mid];
-      if (v == (int32_t)r) { found = true; break; }
-      if (v < (int32_t)r) lo = mid + 1; else hi = mid;
+    while (lo < hi) {  // lower bound of r in row c
+      const int32_t mid = (lo + hi) >> 1;
+      if (cols[mid] < (int32_t)r) lo = mid + 1; else hi = mid;
     }
-    if (!found) { flags[0] = 0; return; }
+    int32_t m = lo;
+    hi = row_ptr[c + 1];
+    while (m < hi && cols[m] == (int32_t)r) ++m;
+    if (m - lo != q - p) { flags[0] = 0; return; }
+    p = q;
   }
 }
 
