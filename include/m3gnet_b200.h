@@ -475,6 +475,43 @@ int m3g_fire_step(const float* forces, const float* sigma, const float* energy, 
                   void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Batched Langevin MD (csrc/md.cu; extension, no reference counterpart): BAOAB (Leimkuhler & Matthews 2013) on fixed
+ * cells for every running structure of a ragged batch.  Positions pos (N,3) f64 A, velocities v (N,3) f64 A/fs,
+ * inv_mass (N) f64 = ACC_UNIT / m (calculator.py), dt fs; per structure c1 = exp(-gamma dt), c2 = sqrt(1 - c1^2) and
+ * kT (eV) f64, the stream id sid (int64; the structure's index in the caller's list), the step counter step and status
+ * (0 = running, 1 = failed) int32, bath f64.
+ *
+ * Noise: Philox4x64-10 (numpy.random.Philox's generator) with key (seed, 0) (seed reinterpreted as uint64) and counter
+ * (i, sid, k, tag): i = atom index within its structure, k = step, tag 0 = Langevin noise, 1 = starting velocities.
+ * u = ((w >> 11) + 0.5) 2^-53; one call gives xi = (sqrt(-2 ln u0) cos(2 pi u1), sqrt(-2 ln u0) sin(2 pi u1),
+ * sqrt(-2 ln u2) cos(2 pi u3)).  No generator state is stored; the noise names the structure, not its batch row.
+ *
+ * m3g_langevin_step: one launch per MD step with the forces (N,3) and energy (B) f32 of frame k = step[b], for every
+ * structure with status 0:
+ *   1. unless k == 0, the closing half kick v += dt/2 F inv_mass of step k - 1 gives v_k;
+ *   2. the structure fails (status 1; pos, v, step and bath left as they were) if a force, v_k or the energy is not
+ *      finite or max_i |v_k,i| dt > max_step_move; otherwise, when slot >= 0, obs[slot, b, :] (f64) =
+ *      (E_pot, E_kin, T_kin = 2 E_kin / ((3 n_b - 3) kB), bath) with E_kin = sum |v_k|^2 / (2 inv_mass);
+ *   3. advance != 0: B (v += dt/2 F inv_mass), A (x += dt/2 v), O (v = c1 v + c2 sqrt(kT inv_mass) xi, counter step k,
+ *      tag 0, then the mass-weighted mean velocity removed), A (x += dt/2 v) -> x_{k+1}; bath += the kinetic energy the
+ *      O step and the removal added; step = k + 1.  advance == 0 (the final frame): v = v_k.
+ * One 256-thread block per structure; every sum runs in relax.cu's fixed thread-row map and tree (no atomics, no
+ * scratch), so a structure's new state depends only on its own rows and sid.
+ *
+ * m3g_md_maxwell_boltzmann: v = sqrt(kT inv_mass) xi (counter step 0, tag 1), then the mass-weighted mean velocity of
+ * each structure removed; no rescaling.  One launch, one block per structure.
+ *
+ * m3g_debug_philox4x64: out (n,4) = philox4x64_10(ctr (n,4), key (n,2)), words as uint64 in int64 storage.
+ * ------------------------------------------------------------------------------------------- */
+int m3g_langevin_step(const float* forces, const float* energy, const int32_t* atom_ptr, int64_t B, double dt,
+                      double max_step_move, int64_t seed, int advance, int slot, const double* inv_mass,
+                      const double* c1, const double* c2, const double* kT, const int64_t* sid, double* pos, double* v,
+                      int32_t* step, int32_t* status, double* bath, double* obs, void* stream);
+int m3g_md_maxwell_boltzmann(const int32_t* atom_ptr, int64_t B, int64_t seed, const double* inv_mass,
+                             const double* kT, const int64_t* sid, double* v, void* stream);
+int m3g_debug_philox4x64(const int64_t* ctr, const int64_t* key, int64_t n, int64_t* out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Domain decomposition helpers (new; nothing in the reference — nn/gradient.py:26 TODO)
  * ------------------------------------------------------------------------------------------- */
 /* out[r] = in[idx[r]] rows of width W floats (halo pack) ; in[idx[r]] += add[r] (reverse halo unpack) */

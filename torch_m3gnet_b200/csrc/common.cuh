@@ -60,6 +60,34 @@ __device__ __forceinline__ float group_sum(float v) {
   return v;
 }
 
+// Fixed-order float64 reductions of the one-block-per-structure kernels (relax.cu, md.cu): xor butterfly in each warp,
+// then the kWarps warp results in warp order; every thread gets the result.  sh holds kWarps doubles.
+template <int kWarps>
+__device__ __forceinline__ double block_sum(double t, double* sh) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(FULL, t, o);
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
+  __syncthreads();
+  double s = 0.0;
+#pragma unroll
+  for (int q = 0; q < kWarps; ++q) s += sh[q];
+  __syncthreads();  // sh is reused by the next reduction
+  return s;
+}
+
+template <int kWarps>
+__device__ __forceinline__ double block_max(double t, double* sh) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t = fmax(t, __shfl_xor_sync(FULL, t, o));
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
+  __syncthreads();
+  double s = sh[0];
+#pragma unroll
+  for (int q = 1; q < kWarps; ++q) s = fmax(s, sh[q]);
+  __syncthreads();
+  return s;
+}
+
 // cutoff polynomial of nn/interaction.py:389-400 and its derivative w.r.t. r
 __device__ __forceinline__ float cutoff_poly(float r, float r3) {
   float x = r / r3;

@@ -25,30 +25,6 @@ struct FireArgs {
   double *lattice, *pos, *fmax, *e_frame, *sigma_frame;
 };
 
-__device__ __forceinline__ double block_sum(double t, double* sh) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(FULL, t, o);
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
-  __syncthreads();
-  double s = 0.0;
-#pragma unroll
-  for (int q = 0; q < kFireWarps; ++q) s += sh[q];
-  __syncthreads();  // sh is reused by the next reduction
-  return s;
-}
-
-__device__ __forceinline__ double block_max(double t, double* sh) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) t = fmax(t, __shfl_xor_sync(FULL, t, o));
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = t;
-  __syncthreads();
-  double s = sh[0];
-#pragma unroll
-  for (int q = 1; q < kFireWarps; ++q) s = fmax(s, sh[q]);
-  __syncthreads();
-  return s;
-}
-
 // inverse of a row-major 3x3 matrix (adjugate / determinant)
 __device__ void inverse3(const double* m, double* inv) {
   const double c00 = m[4] * m[8] - m[5] * m[7], c01 = m[5] * m[6] - m[3] * m[8], c02 = m[3] * m[7] - m[4] * m[6];
@@ -143,10 +119,10 @@ __global__ void __launch_bounds__(kFireThreads) fire_step_kernel(FireArgs p) {
     bad |= !(isfinite(g[0]) && isfinite(g[1]) && isfinite(g[2]));
   }
   bad = __syncthreads_or(bad);
-  P = block_sum(P, sh);
-  gg = block_sum(gg, sh);
-  vv = block_sum(vv, sh);
-  gmax2 = block_max(gmax2, sh);
+  P = block_sum<kFireWarps>(P, sh);
+  gg = block_sum<kFireWarps>(gg, sh);
+  vv = block_sum<kFireWarps>(vv, sh);
+  gmax2 = block_max<kFireWarps>(gmax2, sh);
 
   if (tid == 0) {
     const double fm = sqrt(gmax2);
@@ -205,7 +181,7 @@ __global__ void __launch_bounds__(kFireThreads) fire_step_kernel(FireArgs p) {
       dr2 += d * d;
     }
   }
-  const double norm = sqrt(block_sum(dr2, sh));
+  const double norm = sqrt(block_sum<kFireWarps>(dr2, sh));
   const bool clip = norm > p.max_move;
   const double scale = clip ? p.max_move / norm : 1.0;
   auto step_of = [&](double w) { const double d = dt * w; return clip ? d * scale : d; };
