@@ -498,6 +498,24 @@ int m3g_fire_step(const float* forces, const float* sigma, const float* energy, 
  * One 256-thread block per structure; every sum runs in relax.cu's fixed thread-row map and tree (no atomics, no
  * scratch), so a structure's new state depends only on its own rows and sid.
  *
+ * m3g_langevin_npt_step: m3g_langevin_step plus a stochastic cell-rescaling barostat (Bernetti & Bussi 2020), same
+ * kernel body.  Extra inputs: the cell stress sigma (B,3,3) f32 of frame k (eV/A^3, ASE sign, P = -tr sigma / 3), the
+ * lattice (B,3,3) f64 row-major (rows are lattice vectors; L_k in, L_{k+1} out), per structure P0 (eV/A^3), beta_T
+ * (A^3/eV) and tau_p (fs) f64, coupling (0 = isotropic, 1 = per Cartesian axis) and max_step_strain.  After step 1:
+ *   - V = |det L_k|, P_int = 2 E_kin / (3 V) - tr(sigma) / 3, per axis P_a = 2 K_aa / V - sigma_aa with
+ *     K_aa = sum v_a^2 / (2 inv_mass);
+ *   - d eps = -(beta_T dt / tau_p) (P0 - P) + sqrt(2 kT beta_T dt / (V tau_p)) xi with xi from counter
+ *     (0, sid, k, tag 2): one step in ln V with P = P_int and xi_0 (isotropic, mu_a = exp(d eps / 3)), or one per axis
+ *     with P = P_a and xi_a (mu_a = exp(d eps_a));
+ *   - the structure also fails if an entry of sigma or V is not finite or any |ln mu_a| > max_step_strain (lattice left
+ *     as it was too);
+ *   - obs rows are (E_pot, E_kin, T_kin, bath, V, P_int), 6 columns isotropic, and per axis 9 with (P_x, P_y, P_z)
+ *     appended: obs is (n_slots, B, 6) or (n_slots, B, 9);
+ *   - advance != 0: after B A O A, x_{k+1} = x_{k+1} diag(mu), v = v diag(mu)^-1, L_{k+1} = L_k diag(mu).  bath keeps
+ *     its meaning (the O step and the centre-of-mass removal; the barostat's work is not in it).
+ * With beta_T = 0, mu = 1 exactly and pos, v, step, status, bath and obs[..., :4] are bitwise those of
+ * m3g_langevin_step.
+ *
  * m3g_md_maxwell_boltzmann: v = sqrt(kT inv_mass) xi (counter step 0, tag 1), then the mass-weighted mean velocity of
  * each structure removed; no rescaling.  One launch, one block per structure.
  *
@@ -507,6 +525,12 @@ int m3g_langevin_step(const float* forces, const float* energy, const int32_t* a
                       double max_step_move, int64_t seed, int advance, int slot, const double* inv_mass,
                       const double* c1, const double* c2, const double* kT, const int64_t* sid, double* pos, double* v,
                       int32_t* step, int32_t* status, double* bath, double* obs, void* stream);
+int m3g_langevin_npt_step(const float* forces, const float* energy, const int32_t* atom_ptr, int64_t B, double dt,
+                          double max_step_move, int64_t seed, int advance, int slot, const double* inv_mass,
+                          const double* c1, const double* c2, const double* kT, const int64_t* sid, double* pos,
+                          double* v, int32_t* step, int32_t* status, double* bath, double* obs, const float* sigma,
+                          double* lattice, const double* P0, const double* beta_T, const double* tau_p, int coupling,
+                          double max_step_strain, void* stream);
 int m3g_md_maxwell_boltzmann(const int32_t* atom_ptr, int64_t B, int64_t seed, const double* inv_mass,
                              const double* kT, const int64_t* sid, double* v, void* stream);
 int m3g_debug_philox4x64(const int64_t* ctr, const int64_t* key, int64_t n, int64_t* out, void* stream);

@@ -1,6 +1,7 @@
 // Batched Langevin molecular dynamics (extension, no reference counterpart; torch_m3gnet_b200/md.py::BatchMD): one
-// BAOAB step for every running structure of a ragged batch, the Maxwell-Boltzmann draw of starting velocities, and the
-// counter-based Philox4x64-10 generator both take their noise from.
+// BAOAB step for every running structure of a ragged batch, optionally with a stochastic cell-rescaling barostat
+// (Bernetti & Bussi 2020) for constant pressure, the Maxwell-Boltzmann draw of starting velocities, and the
+// counter-based Philox4x64-10 generator all of them take their noise from.
 //
 // One CTA per structure with relax.cu's thread-row map (thread t owns atoms t, t + 256, ... of its structure) and its
 // fixed reduction tree (block_sum / block_max, common.cuh).  The noise of atom i is keyed to (i, the structure's stream
@@ -15,7 +16,8 @@ constexpr int kMdWarps = kMdThreads / 32;
 constexpr double kBoltzmann = 8.617333262e-5;  // eV/K
 
 enum MdStatus { kMdRunning = 0, kMdFailed = 1 };
-enum NoiseTag : uint64_t { kTagLangevin = 0, kTagVelocities = 1 };
+enum NoiseTag : uint64_t { kTagLangevin = 0, kTagVelocities = 1, kTagBarostat = 2 };
+enum Coupling { kIsotropic = 0, kPerAxis = 1 };
 
 // Philox4x64-10 (Salmon et al., SC'11; Random123's philox4x64, numpy.random.Philox): ten rounds on the counter c, the
 // key bumped by the Weyl constants before every round but the first
@@ -69,11 +71,63 @@ struct LangevinArgs {
   double *bath, *obs;
 };
 
-__global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs p) {
+// the barostat's inputs (m3g_langevin_npt_step); not read by the fixed-cell instance
+struct BarostatArgs {
+  const float* sigma;  // (B,3,3) cell stress of frame k, eV/A^3, ASE sign
+  double* lattice;     // (B,3,3) row-major, rows are lattice vectors; L_k in, L_{k+1} out
+  const double *P0, *beta_T, *tau_p;
+  int coupling;
+  double max_step_strain;
+};
+
+// Stochastic cell rescaling on thread 0 after pass 1: V = |det L|, the pressure P_int = 2 K / (3 V) - tr(sigma) / 3 (and
+// per axis P_a = 2 K_aa / V - sigma_aa), and the log-strain step of Ito Euler-Maruyama in ln V (isotropic) or in the
+// log axis scales (per axis), d eps = -(beta_T dt / tau_p) (P0 - P) + sqrt(2 kT beta_T dt / (V tau_p)) xi with xi from
+// counter (0, s, k, tag 2).  mu = the axis scale factors.  False (the structure fails) on a non-finite stress or volume or
+// a log-scale step beyond max_step_strain.
+__device__ bool barostat(const BarostatArgs& q, int64_t b, double ek, const double ka[3], double kT, double dt,
+                         uint64_t s, uint64_t k, uint64_t seed, double* vol, double* pint, double pa[3],
+                         double mu[3]) {
+  const double* L = q.lattice + b * 9;
+  const float* sg = q.sigma + b * 9;
+  bool ok = true;
+#pragma unroll
+  for (int i = 0; i < 9; ++i) ok &= isfinite(sg[i]);
+  const double V = fabs(L[0] * (L[4] * L[8] - L[5] * L[7]) - L[1] * (L[3] * L[8] - L[5] * L[6]) +
+                        L[2] * (L[3] * L[7] - L[4] * L[6]));
+  const double s00 = sg[0], s11 = sg[4], s22 = sg[8];
+  *vol = V;
+  *pint = 2.0 * ek / (3.0 * V) - (s00 + s11 + s22) / 3.0;
+  pa[0] = 2.0 * ka[0] / V - s00;
+  pa[1] = 2.0 * ka[1] / V - s11;
+  pa[2] = 2.0 * ka[2] / V - s22;
+  double xi[3];
+  normal3(0, s, k, kTagBarostat, seed, xi);
+  const double P0 = q.P0[b], drift = q.beta_T[b] * dt / q.tau_p[b];
+  const double diff = sqrt(2.0 * kT * q.beta_T[b] * dt / (V * q.tau_p[b]));
+  double le[3];
+  if (q.coupling == kIsotropic) {
+    le[0] = le[1] = le[2] = (-drift * (P0 - *pint) + diff * xi[0]) / 3.0;
+  } else {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) le[a] = -drift * (P0 - pa[a]) + diff * xi[a];
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    ok &= fabs(le[a]) <= q.max_step_strain;  // false on NaN too
+    mu[a] = exp(le[a]);
+  }
+  return ok && isfinite(V);
+}
+
+// kNpt: with the barostat (BarostatArgs); otherwise the fixed-cell step, which reads nothing of q
+template <bool kNpt>
+__global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs p, BarostatArgs q) {
   const int64_t b = blockIdx.x;
   if (p.status[b] != kMdRunning) return;  // failed structures stay frozen at the frame that failed
   __shared__ double sh[kMdWarps];
   __shared__ double vcom[3];
+  __shared__ double mu[3], rmu[3];  // barostat scale factors and their inverses
   __shared__ int bgo;
   const int64_t r0 = p.atom_ptr[b];
   const int n = p.atom_ptr[b + 1] - p.atom_ptr[b];
@@ -89,8 +143,9 @@ __global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs 
     for (int c = 0; c < 3; ++c) w[c] = closing ? v[c] + h * ((double)f[c] * im) : v[c];
   };
 
-  // pass 1: v_k, finiteness, max |v_k|^2, kinetic energy and total mass (in units of 1 / ACC_UNIT)
-  double ek = 0.0, vmax2 = 0.0, mass = 0.0;
+  // pass 1: v_k, finiteness, max |v_k|^2, kinetic energy (and per axis with the barostat) and total mass (in units of
+  // 1 / ACC_UNIT)
+  double ek = 0.0, vmax2 = 0.0, mass = 0.0, ka[3] = {0.0, 0.0, 0.0};
   int bad = 0;
   for (int r = tid; r < n; r += kMdThreads) {
     const float* f = p.forces + (r0 + r) * 3;
@@ -100,6 +155,12 @@ __global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs 
     const double w2 = w[0] * w[0] + w[1] * w[1] + w[2] * w[2];
     bad |= !(isfinite(f[0]) && isfinite(f[1]) && isfinite(f[2]) && isfinite(w2));
     ek += w2 / im;
+    if constexpr (kNpt) {
+#pragma unroll
+      // (w / im) w, not w w / im: a shared w w product would let the compiler rebuild w2 without its fmas and move
+      // E_kin off the fixed-cell step's bits
+      for (int c = 0; c < 3; ++c) ka[c] += (w[c] / im) * w[c];
+    }
     vmax2 = fmax(vmax2, w2);
     mass += 1.0 / im;
   }
@@ -107,18 +168,49 @@ __global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs 
   ek = 0.5 * block_sum<kMdWarps>(ek, sh);
   vmax2 = block_max<kMdWarps>(vmax2, sh);
   mass = block_sum<kMdWarps>(mass, sh);
+  if constexpr (kNpt) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) ka[c] = 0.5 * block_sum<kMdWarps>(ka[c], sh);
+  }
 
   if (tid == 0) {
     const double e = (double)p.energy[b];
-    const bool fail = bad || !isfinite(e) || !(sqrt(vmax2) * p.dt <= p.max_step_move);
+    bool fail = bad || !isfinite(e) || !(sqrt(vmax2) * p.dt <= p.max_step_move);
+    double vol = 0.0, pint = 0.0, pa[3], m[3];
+    if constexpr (kNpt) {
+      fail |= !barostat(q, b, ek, ka, p.kT[b], p.dt, (uint64_t)p.sid[b], (uint64_t)k, p.seed, &vol, &pint, pa, m);
+    }
     if (fail) {
       p.status[b] = kMdFailed;
     } else if (p.slot >= 0) {
-      double* o = p.obs + ((int64_t)p.slot * p.B + b) * 4;
+      // obs rows: 4 columns fixed-cell; with the barostat 6 (+ V, P_int), per axis 9 (+ P_x, P_y, P_z)
+      const int width = !kNpt ? 4 : q.coupling == kIsotropic ? 6 : 9;
+      double* o = p.obs + ((int64_t)p.slot * p.B + b) * width;
       o[0] = e;
       o[1] = ek;
       o[2] = 2.0 * ek / ((3.0 * n - 3.0) * kBoltzmann);
       o[3] = p.bath[b];
+      if constexpr (kNpt) {
+        o[4] = vol;
+        o[5] = pint;
+        if (q.coupling != kIsotropic) {
+          o[6] = pa[0];
+          o[7] = pa[1];
+          o[8] = pa[2];
+        }
+      }
+    }
+    if constexpr (kNpt) {
+      if (!fail && p.advance) {  // L_{k+1} = L_k diag(mu)
+        double* L = q.lattice + b * 9;
+#pragma unroll
+        for (int i = 0; i < 9; ++i) L[i] *= m[i % 3];
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+          mu[a] = m[a];
+          rmu[a] = 1.0 / m[a];
+        }
+      }
     }
     bgo = !fail;
   }
@@ -175,7 +267,8 @@ __global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs 
   }
   __syncthreads();
 
-  // pass 3: centre-of-mass velocity removed, A (x + dt/2 v) -> x_{k+1}; kinetic energy after the thermostat
+  // pass 3: centre-of-mass velocity removed, A (x + dt/2 v) -> x_{k+1}; kinetic energy after the thermostat (before the
+  // barostat, which then scales x_{k+1} by mu and v by 1 / mu)
   double ke1 = 0.0;
   for (int r = tid; r < n; r += kMdThreads) {
     const double im = p.inv_mass[r0 + r];
@@ -186,8 +279,13 @@ __global__ void __launch_bounds__(kMdThreads) langevin_step_kernel(LangevinArgs 
     for (int c = 0; c < 3; ++c) {
       const double u = v[c] - vcom[c];
       u2 += u * u;
-      v[c] = u;
-      x[c] = x[c] + h * u;
+      if constexpr (kNpt) {
+        v[c] = u * rmu[c];
+        x[c] = (x[c] + h * u) * mu[c];
+      } else {
+        v[c] = u;
+        x[c] = x[c] + h * u;
+      }
     }
     ke1 += u2 / im;
   }
@@ -269,8 +367,29 @@ int m3g_langevin_step(const float* forces, const float* energy, const int32_t* a
   M3G_REQUIRE(B <= 0x7fffffff, "m3g_langevin_step: B=%lld too large", (long long)B);
   LangevinArgs p{forces, energy, atom_ptr, B, dt, max_step_move, (uint64_t)seed, advance, slot, inv_mass, c1, c2, kT,
                  sid, pos, v, step, status, bath, obs};
-  langevin_step_kernel<<<(unsigned)B, kMdThreads, 0, as_stream(stream)>>>(p);
+  langevin_step_kernel<false><<<(unsigned)B, kMdThreads, 0, as_stream(stream)>>>(p, BarostatArgs{});
   M3G_LAUNCH_CHECK("m3g_langevin_step");
+  return M3G_OK;
+}
+
+int m3g_langevin_npt_step(const float* forces, const float* energy, const int32_t* atom_ptr, int64_t B, double dt,
+                          double max_step_move, int64_t seed, int advance, int slot, const double* inv_mass,
+                          const double* c1, const double* c2, const double* kT, const int64_t* sid, double* pos,
+                          double* v, int32_t* step, int32_t* status, double* bath, double* obs, const float* sigma,
+                          double* lattice, const double* P0, const double* beta_T, const double* tau_p, int coupling,
+                          double max_step_strain, void* stream) {
+  if (B == 0) return M3G_OK;
+  M3G_REQUIRE(forces && energy && atom_ptr && inv_mass && c1 && c2 && kT && sid && pos && v && step && status && bath &&
+                  sigma && lattice && P0 && beta_T && tau_p,
+              "m3g_langevin_npt_step: null pointer");
+  M3G_REQUIRE(slot < 0 || obs, "m3g_langevin_npt_step: slot %d needs obs", slot);
+  M3G_REQUIRE(coupling == kIsotropic || coupling == kPerAxis, "m3g_langevin_npt_step: coupling %d", coupling);
+  M3G_REQUIRE(B <= 0x7fffffff, "m3g_langevin_npt_step: B=%lld too large", (long long)B);
+  LangevinArgs p{forces, energy, atom_ptr, B, dt, max_step_move, (uint64_t)seed, advance, slot, inv_mass, c1, c2, kT,
+                 sid, pos, v, step, status, bath, obs};
+  BarostatArgs q{sigma, lattice, P0, beta_T, tau_p, coupling, max_step_strain};
+  langevin_step_kernel<true><<<(unsigned)B, kMdThreads, 0, as_stream(stream)>>>(p, q);
+  M3G_LAUNCH_CHECK("m3g_langevin_npt_step");
   return M3G_OK;
 }
 
