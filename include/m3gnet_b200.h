@@ -475,6 +475,35 @@ int m3g_fire_step(const float* forces, const float* sigma, const float* energy, 
                   void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Batched climbing-image NEB step (csrc/neb.cu; extension, no reference counterpart): one FIRE step of every running
+ * band of a ragged batch, improved tangent (Henkelman & Jonsson 2000) with an optional climbing image, as ASE's
+ * NEB(method="improvedtangent") optimised by FIRE.  Band b has M_b = image_ptr[b+1] - image_ptr[b] interior images
+ * (1 <= M_b <= M3G_NEB_MAX_IMAGES) of n_b = (end_ptr[b+1] - end_ptr[b]) / 2 atoms each: interior rows row_ptr[b] ..
+ * row_ptr[b+1] (= M_b n_b rows, image-major) of pos / v / forces (f64 / f64 / f32, (rows,3)), interior energies
+ * energy[image_ptr[b] ..] f32, endpoint positions ends rows end_ptr[b] .. (image 0's n_b rows, then image M_b+1's)
+ * and endpoint energies e_end (B,2) f64, spring constant k[b] (eV/A^2).  For every band with status[b] == 0:
+ *   - e_frame[image] = energy (f64); i_climb[b] = the interior image (1 .. M_b, band numbering) of highest energy,
+ *     ties to the lowest index;
+ *   - per interior image i, t+ = R_{i+1} - R_i, t- = R_i - R_{i-1} (raw differences) and the tangent t = t+ if
+ *     E_{i+1} > E_i > E_{i-1}, t- if E_{i+1} < E_i < E_{i-1}, else dVmax t+ + dVmin t- when E_{i+1} > E_{i-1} and
+ *     dVmin t+ + dVmax t- otherwise (dVmax / dVmin = max / min of |E_{i+1} - E_i|, |E_{i-1} - E_i|), t+ + t- when
+ *     dVmax = 0; t^ = t / |t|;
+ *   - G_i = F_i - (F_i.t^) t^ + k (|t+| - |t-|) t^, or F_i - 2 (F_i.t^) t^ for the climbing image when climb != 0;
+ *   - status 3 (failed), fmax = +inf, if an energy is not finite or some |t| is 0 or not finite; otherwise
+ *     m3g_fire_step's fixed-cell step on the band's M_b n_b rows of G as one structure (fmax = max row |G|, power,
+ *     norms and the max_move clip over the band), with dt, a, n_pos, n_steps, status, fmax per band.
+ * Bands with status != 0 are not touched.  max_images: the largest M_b of the launch (checked against the cap).  One
+ * launch, one 256-thread block per band, relax.cu's thread-row map and fixed trees (no atomics, no scratch), so a
+ * band's new state depends only on its own rows. */
+#define M3G_NEB_MAX_IMAGES 64
+int m3g_neb_step(const float* forces, const float* energy, const int32_t* row_ptr, const int32_t* image_ptr,
+                 const int32_t* end_ptr, int64_t B, int max_images, const double* ends, const double* e_end,
+                 const double* k, int climb, double dt_max, double max_move, int n_min, double f_inc, double f_dec,
+                 double a_start, double f_a, double fmax_target, int max_steps, double* pos, double* v, double* dt,
+                 double* a, int32_t* n_pos, int32_t* n_steps, int32_t* status, double* fmax, int32_t* i_climb,
+                 double* e_frame, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Batched Langevin MD (csrc/md.cu; extension, no reference counterpart): BAOAB (Leimkuhler & Matthews 2013) on fixed
  * cells for every running structure of a ragged batch.  Positions pos (N,3) f64 A, velocities v (N,3) f64 A/fs,
  * inv_mass (N) f64 = ACC_UNIT / m (calculator.py), dt fs; per structure c1 = exp(-gamma dt), c2 = sqrt(1 - c1^2) and

@@ -87,7 +87,8 @@ LIB = _Library()
 CALLS = 0
 LAUNCHES = 0
 _KERNELS_PER_CALL = {"exclusive_scan_i32": 3, "csr_by_key": 7, "check_sorted": 2, "csr_is_symmetric": 2,
-                     "forces_virial": 2, "bond_virial": 2, "fire_step": 1}
+                     "forces_virial": 2, "bond_virial": 2, "fire_step": 1,
+                     "neb_step": 1}
 # when set to a dict, every call is bracketed by CUDA events on the launching stream: {name: [(start, end), ...]}
 PROFILE = None
 

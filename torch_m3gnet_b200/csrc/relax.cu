@@ -4,14 +4,9 @@
 // (thread t owns rows t, t + 256, ... counted from the structure's first row) and every sum ends in the same fixed tree
 // (xor butterfly in each warp, then the 8 warp results in warp order).  The result therefore depends only on the
 // structure's own rows, never on its offset in the batch or its neighbours, and there are no atomics.
-#include "common.cuh"
+#include "fire.cuh"
 
 namespace m3g {
-
-constexpr int kFireThreads = 256;
-constexpr int kFireWarps = kFireThreads / 32;
-
-enum FireStatus { kFireRunning = 0, kFireConverged = 1, kFireNotConverged = 2, kFireFailed = 3 };
 
 struct FireArgs {
   const float *forces, *sigma, *energy;
@@ -51,8 +46,6 @@ __global__ void __launch_bounds__(kFireThreads) fire_step_kernel(FireArgs p) {
   __shared__ double D[9];      // deformation gradient D = solve(L0, L)^T, row-major
   __shared__ double Dn[9];     // D of the updated cell rows, xc / cell_factor
   __shared__ double cellf[9];  // generalised forces of the 3 cell rows
-  __shared__ double bc[5];     // broadcast: 1 - a, a |v|, max(|g|, 1e-30), dt, clip factor
-  __shared__ int bmode;        // 0 = stop, 1 = step with the velocity mix, 2 = step from zero velocity
   const int64_t r0 = p.atom_ptr[b];
   const int n = p.atom_ptr[b + 1] - p.atom_ptr[b];
   const bool cell = p.sigma != nullptr;
@@ -104,87 +97,10 @@ __global__ void __launch_bounds__(kFireThreads) fire_step_kernel(FireArgs p) {
   };
   auto vel = [&](int r) -> double* { return r < n ? p.v + (r0 + r) * 3 : p.vc + b * 9 + (r - n) * 3; };
 
-  // pass 1: power, |g|^2, |v|^2, max row |g|^2, finiteness
-  double P = 0.0, gg = 0.0, vv = 0.0, gmax2 = 0.0;
-  int bad = 0;
-  for (int r = tid; r < rows; r += kFireThreads) {
-    double g[3];
-    gen(r, g);
-    const double* v = vel(r);
-    const double g2 = g[0] * g[0] + g[1] * g[1] + g[2] * g[2];
-    P += g[0] * v[0] + g[1] * v[1] + g[2] * v[2];
-    gg += g2;
-    vv += v[0] * v[0] + v[1] * v[1] + v[2] * v[2];
-    gmax2 = fmax(gmax2, g2);
-    bad |= !(isfinite(g[0]) && isfinite(g[1]) && isfinite(g[2]));
-  }
-  bad = __syncthreads_or(bad);
-  P = block_sum<kFireWarps>(P, sh);
-  gg = block_sum<kFireWarps>(gg, sh);
-  vv = block_sum<kFireWarps>(vv, sh);
-  gmax2 = block_max<kFireWarps>(gmax2, sh);
-
-  if (tid == 0) {
-    const double fm = sqrt(gmax2);
-    p.fmax[b] = bad ? (double)INFINITY : fm;
-    int mode = 0;
-    if (bad) {
-      p.status[b] = kFireFailed;
-    } else if (fm < p.fmax_target) {
-      p.status[b] = kFireConverged;
-    } else if (p.n_steps[b] >= p.max_steps) {
-      p.status[b] = kFireNotConverged;
-    } else {
-      double a = p.a[b], dt = p.dt[b];
-      int n_pos = p.n_pos[b];
-      if (P > 0.0) {
-        mode = 1;
-        bc[0] = 1.0 - a;
-        bc[1] = a * sqrt(vv);
-        bc[2] = fmax(sqrt(gg), 1e-30);
-        if (n_pos > p.n_min) {
-          dt = fmin(dt * p.f_inc, p.dt_max);
-          a *= p.f_a;
-        }
-        n_pos += 1;
-      } else {
-        mode = 2;
-        a = p.a_start;
-        dt *= p.f_dec;
-        n_pos = 0;
-      }
-      p.a[b] = a;
-      p.dt[b] = dt;
-      p.n_pos[b] = n_pos;
-      p.n_steps[b] += 1;
-      bc[3] = dt;
-    }
-    bmode = mode;
-  }
-  __syncthreads();
-  const int mode = bmode;
-  if (mode == 0) return;
-  const double dt = bc[3];
-
-  // pass 2: v <- (1 - a) v + a |v| g / |g|  (or 0), v <- v + dt g; |dr|^2 with dr = dt v
-  double dr2 = 0.0;
-  for (int r = tid; r < rows; r += kFireThreads) {
-    double g[3];
-    gen(r, g);
-    double* v = vel(r);
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      double w = mode == 1 ? bc[0] * v[c] + bc[1] * g[c] / bc[2] : 0.0;
-      w = w + dt * g[c];
-      v[c] = w;
-      const double d = dt * w;
-      dr2 += d * d;
-    }
-  }
-  const double norm = sqrt(block_sum<kFireWarps>(dr2, sh));
-  const bool clip = norm > p.max_move;
-  const double scale = clip ? p.max_move / norm : 1.0;
-  auto step_of = [&](double w) { const double d = dt * w; return clip ? d * scale : d; };
+  const FireParams q{p.dt_max, p.max_move, p.f_inc, p.f_dec, p.a_start, p.f_a, p.fmax_target, p.n_min, p.max_steps};
+  const FireState s{p.dt, p.a, p.fmax, p.n_pos, p.n_steps, p.status};
+  FireMove step_of;
+  if (!fire_advance(q, s, b, rows, gen, vel, sh, &step_of)) return;
 
   // pass 3: x <- x + dr, then back to Cartesian positions and lattice
   if (!cell) {

@@ -57,3 +57,14 @@ def mpf_like_structure(s: int):
         grid = np.stack(np.meshgrid(*[np.arange(m)] * 3, indexing="ij"), axis=-1).reshape(-1, 3)[:n]
         pts = list(((grid + 0.5) / m + rng.uniform(-0.02, 0.02, size=(n, 3))) @ lattice)
     return lattice, np.asarray(pts), rng.choice(species, size=n).astype(np.int64)
+
+
+def fcc_cu_vacancy_hop(reps: int):
+    """(initial, final) of a vacancy hop in reps^3 conventional FCC Cu cells (4 reps^3 - 1 atoms): the vacancy at the
+    origin, and the nearest neighbour at (0, a/2, a/2) moved into it.  Unrelaxed, same atom order in both."""
+    lat, cart, z = fcc_cu_supercell(reps, 0.0, 0)
+    cart, z = cart[1:], z[1:]
+    j = int(np.argmin(np.linalg.norm(cart - np.array([0.0, 0.5, 0.5]) * A_CU, axis=1)))
+    final = cart.copy()
+    final[j] = 0.0
+    return (lat, cart, z), (lat.copy(), final, z.copy())
