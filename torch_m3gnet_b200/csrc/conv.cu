@@ -554,6 +554,7 @@ int m3g_segment_sum_add(const float* base, const float* msg, const int32_t* edge
                         void* stream) {
   if (N == 0) return M3G_OK;
   M3G_REQUIRE(base && msg && edge_ptr && out, "m3g_segment_sum_add: null pointer");
+  M3G_REQUIRE(F >= 1 && F <= M3G_MAX_F, "m3g_segment_sum_add: F=%d outside [1,%d]", F, M3G_MAX_F);
   segment_sum_add_kernel<<<blocks_for(N * 32, 256), 256, 0, as_stream(stream)>>>(base, msg, edge_ptr, N, F, out);
   M3G_LAUNCH_CHECK("m3g_segment_sum_add");
   return M3G_OK;
@@ -602,6 +603,7 @@ int m3g_conv_gather_gz(const float* g_z1, const int32_t* edge_ptr, const int32_t
                        int64_t N, int F, int ldp, int po, float* g_P, void* stream) {
   if (N == 0) return M3G_OK;
   M3G_REQUIRE(g_z1 && edge_ptr && in_ptr && in_perm && g_P, "m3g_conv_gather_gz: null pointer");
+  M3G_REQUIRE(F >= 1 && F <= M3G_MAX_F, "m3g_conv_gather_gz: F=%d outside [1,%d]", F, M3G_MAX_F);
   if (F == 64 && ldp % 4 == 0 && po % 4 == 0)
     conv_gather_gz128_kernel<<<blocks_for(N * 64, 256), 256, 0, as_stream(stream)>>>(g_z1, edge_ptr, in_ptr, in_perm, N,
                                                                                      ldp, po, g_P);

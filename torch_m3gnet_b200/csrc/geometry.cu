@@ -50,10 +50,13 @@ __global__ void angles_bwd_kernel(const float4* __restrict__ vec4, const int64_t
   int64_t e1 = tri[t], e2 = tri[T + t];
   float4 a = vec4[e1];
   float4 b = vec4[e2];
-  float dot = a.x * b.x + a.y * b.y + a.z * b.z;
+  // c rounded exactly as angles_fwd_kernel forms it: the clamp passes the gradient where the forward's unclamped c lies
+  // in [-1, 1] (torch.clamp takes its mask from its input); a contracted dot * (1 / (|a||b|)) can land an ulp across
+  // the bound at collinear bonds
+  float dot = __fadd_rn(__fadd_rn(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y)), __fmul_rn(a.z, b.z));
+  float c = __fdiv_rn(dot, __fmul_rn(a.w, b.w));
+  if (!(c >= -1.0f && c <= 1.0f)) return;
   float inv = 1.0f / (a.w * b.w);
-  float c = dot * inv;
-  if (!(c >= -1.0f && c <= 1.0f)) return;  // clamp passes gradient on the closed interval only
   float g = g_cos[t];
   atomicAdd(&g_vec4[e1 * 4 + 0], g * b.x * inv);
   atomicAdd(&g_vec4[e1 * 4 + 1], g * b.y * inv);
@@ -504,6 +507,8 @@ int m3g_embed_fwd(const float* weight, const int32_t* types, int64_t N, int F, i
 int m3g_edge_adjust_fwd(const float* h, const float* Wt, int64_t E, int R, int F, float* e0, void* stream) {
   if (E == 0) return M3G_OK;
   M3G_REQUIRE(h && Wt && e0, "m3g_edge_adjust_fwd: null pointer");
+  M3G_REQUIRE(R >= 1 && R <= M3G_MAX_RADIAL, "m3g_edge_adjust_fwd: n_max=%d outside [1,%d]", R, M3G_MAX_RADIAL);
+  M3G_REQUIRE(F >= 1 && F <= M3G_MAX_F, "m3g_edge_adjust_fwd: F=%d outside [1,%d]", F, M3G_MAX_F);
   if (F % 4 == 0 && R == 3)
     edge_adjust_fwd4_kernel<3><<<blocks_for(E * (F / 4), 256), 256, 0, as_stream(stream)>>>(h, Wt, E, R, F, e0);
   else if (F % 4 == 0 && R <= 4)
@@ -519,6 +524,7 @@ int m3g_edge_adjust_bwd(const float* h, const float* Wt, const float* g_e0, int6
   if (E == 0) return M3G_OK;
   M3G_REQUIRE(h && Wt && g_e0 && g_h, "m3g_edge_adjust_bwd: null pointer");
   M3G_REQUIRE(R >= 1 && R <= M3G_MAX_RADIAL, "m3g_edge_adjust_bwd: n_max=%d outside [1,%d]", R, M3G_MAX_RADIAL);
+  M3G_REQUIRE(F >= 1 && F <= M3G_MAX_F, "m3g_edge_adjust_bwd: F=%d outside [1,%d]", F, M3G_MAX_F);
   if (F == 64 && R == 3)
     edge_adjust_bwd64_kernel<3><<<blocks_for(E * 16, 256), 256, 0, as_stream(stream)>>>(h, Wt, g_e0, E, R, g_h);
   else if (F == 64 && R <= 4)
