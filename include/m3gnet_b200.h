@@ -504,6 +504,55 @@ int m3g_neb_step(const float* forces, const float* energy, const int32_t* row_pt
                  double* e_frame, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Batched harmonic phonons (csrc/phonon.cu; extension, no reference counterpart).  Structure b has a unit cell of
+ * n_b = atom_ptr[b+1] - atom_ptr[b] atoms (1 <= n_b <= M3G_PHONON_MAX_ATOMS), a diagonal supercell reps[b] (3 int32)
+ * of L_b = r1 r2 r3 cells and N_b = n_b L_b atoms, supercell atom j = l n_b + k' with l = (i1 r2 + i2) r3 + i3.  Its
+ * (k, j) pairs are pair_ptr[b] + k N_b + j; its force constants fc (pairs, 3, 3) f64 eV/A^2 hold
+ * Phi(0k alpha; j beta) (phonopy's compact layout).  Everything is float64 and deterministic: sums run in a fixed
+ * order that depends only on the structure's own data, so its output does not depend on the rest of the batch.
+ *
+ * m3g_phonon_force_constants: forces rows row_ptr[b] .. (f32, (6 n_b + 1) N_b rows: the undisplaced supercell, then
+ *   for k = 0 .. n_b-1 and alpha = x, y, z the supercells with atom k of cell 0 moved by +h and by -h along alpha);
+ *   Phi = -(F(+h) - F(-h)) / 2h, then `symmetrize` rounds of (a) Phi(0k; l k')_ab <- (Phi(0k; l k')_ab +
+ *   Phi(0k'; -l k)_ba) / 2 (-l wrapped in the supercell) and (b) Phi(0k; 0k) -= sum_j Phi(0k; j) (acoustic sum
+ *   rule).  status[b] = 0, residual[b] = max |F| of the undisplaced supercell; a structure with any non-finite force
+ *   gets status 1, NaN force constants and residual.  One 256-thread block per structure.
+ * m3g_phonon_dynmat: dmat (Q, ld, ld) complex128 (re, im interleaved), ld >= 3 max n: D(q) of q-point i (fractional
+ *   coordinates of the unit cell's reciprocal lattice, q (Q,3) f64) of structure b (q_ptr[b] <= i < q_ptr[b+1],
+ *   int32), D_{3k+a, 3k'+b}(q) = sum_l Phi(0k; l k')_ab (1/|M|) sum_{v in M} exp(2 pi i q.v) / sqrt(m_k m_k');
+ *   M is the minimum-image set of the pair: vectors sv[sv_ptr[p] .. sv_ptr[p+1]] (unit-cell fractional coordinates of
+ *   the lattice translation from cell 0 to the image's cell, (rows, 3) f64), sv_ptr (pairs + 1) int64; mass (atoms)
+ *   f64 amu.  Entries outside 3 n_b x 3 n_b are zero.  One block per q-point.
+ * m3g_phonon_frequencies: per q-point the same D(q), its Hermitian part (D + D^H) / 2 and its eigenvalues by a cyclic
+ *   complex Jacobi method (round-robin pair order, 3n/2 disjoint rotations per round), until the off-diagonal
+ *   Frobenius norm is <= 1e-13 ||D||_F.  eig (f64, eV/(amu A^2)) and freq = sign(eig) sqrt(|eig|) thz (THz), ascending,
+ *   at f_ptr[b] + (i - q_ptr[b]) 3 n_b (f_ptr (B+1) int64); sweeps[i] = Jacobi sweeps, q_status[i] = 0.  A structure
+ *   with status[b] != 0, a non-finite D or 30 sweeps without convergence give NaN and q_status 1.  One block per
+ *   q-point, (3 max_atoms)^2 x 16 B of dynamic shared memory.
+ * m3g_phonon_thermal: per structure b and temperature temps[t] (K), over the frequencies f >= cutoff (THz) of its
+ *   q-points with e = h_thz f (eV), x = e / kT, kT = kB T: out[b, t, :] = (F, S, Cv, E) / N_q with
+ *   F = sum e/2 + kT ln(1 - e^-x), S = kB sum x/(e^x - 1) - ln(1 - e^-x), Cv = kB sum x^2 e^x / (e^x - 1)^2,
+ *   E = sum e (1/2 + 1/(e^x - 1)) (T = 0: F = E = sum e/2, S = Cv = 0); n_imag[b] = #{f < -cutoff},
+ *   fmin[b] = min f.  NaN frequencies give NaN; a structure with status[b] != 0 gets NaN, n_imag -1.  One block per
+ *   (structure, temperature); fixed-order block reductions.
+ * ------------------------------------------------------------------------------------------- */
+#define M3G_PHONON_MAX_ATOMS 32
+int m3g_phonon_force_constants(const float* forces, const int64_t* row_ptr, const int32_t* atom_ptr,
+                               const int32_t* reps, const int64_t* pair_ptr, int64_t B, int max_atoms, double h,
+                               int symmetrize, double* fc, int32_t* status, double* residual, void* stream);
+int m3g_phonon_dynmat(const double* fc, const int32_t* atom_ptr, const int32_t* reps, const int64_t* pair_ptr,
+                      const int64_t* sv_ptr, const double* sv, const double* mass, const double* q,
+                      const int32_t* q_ptr, int64_t B, int64_t Q, int max_atoms, int ld, double* dmat, void* stream);
+int m3g_phonon_frequencies(const double* fc, const int32_t* atom_ptr, const int32_t* reps, const int64_t* pair_ptr,
+                           const int64_t* sv_ptr, const double* sv, const double* mass, const int32_t* status,
+                           const double* q, const int32_t* q_ptr, const int64_t* f_ptr, int64_t B, int64_t Q,
+                           int max_atoms, double thz, double* eig, double* freq, int32_t* sweeps, int32_t* q_status,
+                           void* stream);
+int m3g_phonon_thermal(const double* freq, const int64_t* f_ptr, const int32_t* q_ptr, const int32_t* status,
+                       int64_t B, const double* temps, int64_t T, double kB, double h_thz, double cutoff, double* out,
+                       int32_t* n_imag, double* fmin, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Batched Langevin MD (csrc/md.cu; extension, no reference counterpart): BAOAB (Leimkuhler & Matthews 2013) on fixed
  * cells for every running structure of a ragged batch.  Positions pos (N,3) f64 A, velocities v (N,3) f64 A/fs,
  * inv_mass (N) f64 = ACC_UNIT / m (calculator.py), dt fs; per structure c1 = exp(-gamma dt), c2 = sqrt(1 - c1^2) and

@@ -11,3 +11,4 @@ from torch_m3gnet_b200.calculator import Fire, M3GNetCalculator, VelocityVerlet 
 from torch_m3gnet_b200.relax import BatchFire  # noqa: E402,F401
 from torch_m3gnet_b200.md import BatchMD  # noqa: E402,F401
 from torch_m3gnet_b200.neb import BatchNEB  # noqa: E402,F401
+from torch_m3gnet_b200.phonon import BatchPhonon  # noqa: E402,F401
